@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload alarm37] [--precision fp64]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's own CPU implementation, same metric
+    python bench.py ... --dump-outputs DIR    # also write the outputs of the last timed step (rank 0's shard) to DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic evidence cases: init (K0),
 `sweeps` synchronous sweeps (K1), beliefs (K4) -- belief_propagation.hpp:31-159 for every case.
@@ -289,6 +290,26 @@ FMA_PEAK_TFLOPS = {"fp64": 37.2, "fp32": 74.4}     # nominal: 2 x 148 SMs x 1.96
 FP64_TENSOR_PEAK_TFLOPS = 40.0                     # nominal B200 fp64 tensor (DMMA) rate
 
 
+DUMP_BYTES = 60 << 20          # --dump-outputs: bound of the files written (a seeded sample of cases beyond it)
+
+
+def dump_outputs(dirname: str, marginals, sweeps, converged, torch) -> None:
+    """The outputs of the last timed step as DIR/<name>.npy, so that two builds run with the same arguments can be
+    compared output for output: marginals [k, sum r_X] in the handle's precision, the sweeps each case ran and its
+    converged flag (both as float64), and case_index, the cases (rows of the batch) the k rows are.  Every case when
+    that fits DUMP_BYTES, else a fixed sample drawn with a fixed seed."""
+    n, V = marginals.shape
+    row_bytes = V * marginals.element_size() + 3 * 8
+    k = min(n, DUMP_BYTES // row_bytes)
+    rows = np.arange(n) if k == n else np.sort(np.random.default_rng(20240).choice(n, k, replace=False))
+    idx = torch.from_numpy(rows).to(marginals.device)
+    out = {"marginals": marginals[idx].cpu().numpy(), "sweeps": sweeps[idx].cpu().numpy().astype(np.float64),
+           "converged": converged[idx].cpu().numpy().astype(np.float64), "case_index": rows.astype(np.float64)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def walk_flops(net) -> float:
     """F = sum_X (2k+2) r_X Q_X: one fused CPT pass for pi_X and all k lambda-messages (SURVEY.md 8d)."""
     k = np.diff(net.parent_off).astype(np.float64)
@@ -442,7 +463,8 @@ def measure_config(key, workload, total_cases, base_gpus, precision, parity_case
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline measurement (the e2e leg times min(K, 10) calls, the N > 1 gather pass max(3, K // 2) steps, each `configs` entry 1 or 2 steps of its own)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="bnbp", choices=["bnbp", "reference"])
     ap.add_argument("--workload", default="alarm37", choices=sorted(synth.WORKLOADS))
@@ -469,7 +491,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true",
                     help="skip the short measured entries for BASELINE configs 3-5 (the `configs` array of the line)")
     ap.add_argument("--only-configs", default="", help="comma-separated subset of cfg3,cfg4,cfg5")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the marginals, sweeps and converged flags of the last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path: it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "bnbp" else args.warmup
 
     if os.environ.get("BNBP_BENCH_WATCHDOG"):
@@ -593,6 +621,10 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     st = bp.stats()
+    if args.dump_outputs:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, d_out, d_sw, d_cv, torch)
+        barrier()                                    # rank 0 allocates for the copy: no peer may sit in a collective meanwhile
     gather_pass = None
     if gather:
         # the same step with the gather of the marginals inside the call (every rank ends it with ALL marginals)

@@ -5,7 +5,10 @@
 
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
 #include <fstream>
+
+#include <unistd.h>
 
 #include "bayesian/graph.hpp"
 #include "bayesian/inference/belief_propagation.hpp"
@@ -85,7 +88,11 @@ BOOST_AUTO_TEST_CASE(sampler_make_cpt_counts_on_the_device)
     BOOST_CHECK((b->cpt[{{a, 0}}].second == std::vector<double>{5.0 / 6.0, 1.0 / 6.0}));
     BOOST_CHECK((b->cpt[{{a, 1}}].second == std::vector<double>{0.0, 1.0}));
     // the reference's sample-file format: "count s_0 s_1" per line
-    char const* path = "/tmp/bnbp_test_samples.txt";
+    // (a file of its own: on a shared machine a fixed name under /tmp may belong to another user)
+    char path[] = "/tmp/bnbp_test_samples_XXXXXX";
+    const int fd = mkstemp(path);
+    BOOST_CHECK(fd >= 0);
+    if (fd >= 0) close(fd);
     { std::ofstream f(path); f << "3 0 0\n1 0 1\n"; }
     bn::sampler from_file(path);
     BOOST_CHECK(from_file.load_sample(g.vertex_list()));
