@@ -1880,9 +1880,13 @@ int build_layout(const bnbp_flat_network* net, const bnbp_options* opt, bnbp_han
         h->oc_ahead = 1;
         if (const char* ev = getenv("BNBP_OC_AHEAD")) h->oc_ahead = std::min(4, std::max(0, atoi(ev)));
         h->oc_smem = onchip_smem_bytes(L, h->precision == BNBP_FP32, h->oc_roles);
-        h->oc_eligible = h->spec_eligible_ && !h->spec_classloop && h->oc_smem <= SMEM_OPTIN;
+        int max_children = 0;
+        for (int x = 0; x < h->N; ++x) max_children = std::max(max_children, (int)h->nodes[x].m);
+        h->oc_eligible = h->spec_eligible_ && !h->spec_classloop && max_children <= ONCHIP_MREG && h->oc_smem <= SMEM_OPTIN;
         if (!h->spec_eligible_) h->oc_why = h->spec_why;
         else if (h->spec_classloop) h->oc_why = "the network is walked class by class (the on-chip kernel unrolls the walk node by node)";
+        else if (max_children > ONCHIP_MREG)
+            h->oc_why = "a hub with more than " + std::to_string(ONCHIP_MREG) + " children: its inbox cannot be read before the sweep barrier";
         else if (!h->oc_eligible) h->oc_why = "the state of 32 cases (" + std::to_string(h->oc_smem) + " B) exceeds the shared memory of an SM";
         h->oc_minb = (int)std::max<size_t>(1, std::min<size_t>(8, (228 * 1024) / (h->oc_smem + 1024)));
         if (const char* ev = getenv("BNBP_OC_MINB")) h->oc_minb = std::min(16, std::max(1, atoi(ev)));

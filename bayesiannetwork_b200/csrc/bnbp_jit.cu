@@ -289,6 +289,7 @@ std::string spec_source(const SpecLayout& L, const SpecConfig& cfg)
         table("unsigned char", "bnbp_cardn", [&](int x) { return (int)L.nodes[x].card; });
         s << "#define BNBP_WALK\n";
         s << kSpecHeader << "\n" << kOnchipHeader;
+        s << "\nstatic_assert(bnbp_spec::MREG == " << ONCHIP_MREG << ", \"on-chip eligibility (ONCHIP_MREG) and the kernel's MREG disagree\");\n";
         return s.str();
     }
     // walk: declarations, then loads `ahead` nodes in front of the arithmetic

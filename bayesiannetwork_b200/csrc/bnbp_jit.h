@@ -45,6 +45,12 @@ std::vector<int> spec_partition(const SpecLayout& L, int roles, double* imbalanc
 // bytes of dynamic shared memory the on-chip kernel needs for one 32-case group
 size_t onchip_smem_bytes(const SpecLayout& L, bool fp32, int roles);
 
+// Children whose lambda-messages the on-chip kernel reads into registers in phase A, before the sweep barrier
+// (bnbp_spec.cuh MREG; the generated on-chip source static_asserts that the two agree).  A node with more children
+// would read its inbox in phase B, after other warps may have overwritten it with the next sweep's messages: such a
+// network is not eligible for the on-chip kernel.
+constexpr int ONCHIP_MREG = 64;
+
 // Can (and should) this network be specialised?  why != nullptr receives the reason when not.
 bool spec_eligible(const SpecLayout& L, bool fp32, std::string* why);
 

@@ -51,6 +51,19 @@ def jobs():
     out.append((synth.alarm37(), "fp64", 0b11101, force))
     out.append((synth.grid(100), "fp64", 0b11101))
     out.append((synth.grid(100), "fp32", 0b11001))
+    # the shape-boundary networks (tests/test_gpu_edge_shapes.py): unrolled walks (fused variants included), class-looped
+    # walks, the on-chip kernel (fixed / epsilon in fp64, double marginals from a float kernel; refused for hub65: reported
+    # as not compiled), and hub65 the way AUTO lays it out
+    import edge_networks as en
+    unrolled = {"BNBP_CLASSLOOP": "0"}
+    for net in en.catalogue().values():
+        out.append((net, "fp64", 0b01111111, unrolled))
+        out.append((net, "fp32", 0b11111111, unrolled))
+        out.append((net, "fp64", 0b11111, force))
+        out.append((net, "fp32", 0b11111, force))
+        out.append((net, "fp64", (1 << 8) | (1 << 10), unrolled))
+        out.append((net, "fp32", 1 << 9, unrolled))
+    out.append((en.catalogue()["hub65"], "fp64", 0b01111111))
     return out
 
 

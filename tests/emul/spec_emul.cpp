@@ -18,6 +18,31 @@ int emul_value_bytes() { return (int)sizeof(T); }
 
 void emul_set_cpt(const T* cpt, long long n) { memcpy(bnbp_cpt, cpt, (size_t)n * sizeof(T)); }
 
+// What the kernel keeps in registers, per node of the walk (unrolled) or per node class (class-looped), in walk order:
+// children whose lambda-messages are loaded ahead (0: streamed where used) and CPT entries loaded ahead (0: read where
+// used).  The generator's register budget (class_inputs in bnbp_jit.cu) assumes the same split.  Returns the count.
+int emul_register_plan(int* children, int* cpt)
+{
+    int n = 0;
+    auto rec = [&](int m, bool reg_children, bool reg_cpt, int nq) {
+        children[n] = (m > 0 && reg_children) ? m : 0;
+        cpt[n] = reg_cpt ? nq : 0;
+        ++n;
+    };
+    (void)rec;
+#define BNBP_PLAN(NN) rec(NN::M, NN::M <= bnbp_spec::MREG, bnbp_spec::In<NN>::CPT_REG, bnbp_spec::In<NN>::NQ);
+#if BNBP_CLASSLOOP
+#define BNBP_CLASS(CC, FIRST, COUNT) BNBP_PLAN(CC)
+#else
+#define BNBP_DECL(NN) BNBP_PLAN(NN)
+#define BNBP_LOAD(NN)
+#define BNBP_COMP(NN)
+#define BNBP_FLUSH(J0, WW)
+#endif
+    BNBP_WALK
+    return n;
+}
+
 // One launch of <<<(tiles, node_slices), 128>>> bnbp_spec_sweep(pl, cur, nxt, evbits, aux).  delta / status / sweeps / last_active: the
 // per-case arrays of the freeze / check variants (ignored by the plain ones).  evst: variant 5 only.
 void emul_launch(T* pl, const T* cur, T* nxt, const unsigned* evbits, int tiles, int n_inner, T eps, T damping,

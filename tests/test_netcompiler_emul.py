@@ -11,6 +11,7 @@ import ctypes as C
 import os
 import shutil
 import subprocess
+import threading
 
 import numpy as np
 import pytest
@@ -20,7 +21,25 @@ from bayesiannetwork_b200.flat import EvidenceBatch
 from helpers import assert_close
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+# the generator reads its knobs from the environment: one source generation at a time, so that kernels can be built
+# from several threads (the g++ runs are what takes the time)
+SOURCE_LOCK = threading.Lock()
 pytestmark = pytest.mark.skipif(shutil.which("g++") is None, reason="g++ not available")
+
+
+def generated_source(engine, net, precision, variant, env):
+    """engine.spec_source with generator knobs (BNBP_CLASSLOOP, BNBP_OC_ROLES, ...) set in the environment meanwhile."""
+    with SOURCE_LOCK:
+        saved = {k: os.environ.get(k) for k in env}
+        os.environ.update(env)
+        try:
+            return engine.spec_source(net, precision, variant)
+        finally:
+            for k, v in saved.items():
+                if v is None:
+                    del os.environ[k]
+                else:
+                    os.environ[k] = v
 
 
 @pytest.fixture(scope="module")
@@ -34,12 +53,7 @@ class Emulated:
     """One generated kernel (network x precision x variant x walk mode) as a host shared object."""
 
     def __init__(self, engine, net, precision, variant, classloop, workdir, vec=1):
-        os.environ["BNBP_CLASSLOOP"] = "2" if classloop else "0"
-        os.environ["BNBP_SPEC_VEC"] = str(vec)
-        try:
-            src = engine.spec_source(net, precision, variant)
-        finally:
-            del os.environ["BNBP_CLASSLOOP"], os.environ["BNBP_SPEC_VEC"]
+        src = generated_source(engine, net, precision, variant, {"BNBP_CLASSLOOP": "2" if classloop else "0", "BNBP_SPEC_VEC": str(vec)})
         assert ("#define BNBP_CLASSLOOP 1" in src) == classloop
         tag = f"{net.name}_{precision}_v{variant}_{'cls' if classloop else 'unr'}_x{vec}"
         cu = os.path.join(workdir, tag + ".cu")

@@ -14,6 +14,7 @@ import pytest
 
 from bayesiannetwork_b200 import synth
 from helpers import assert_close
+from test_netcompiler_emul import generated_source
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 pytestmark = pytest.mark.skipif(shutil.which("g++") is None, reason="g++ not available")
@@ -31,12 +32,14 @@ def engine():
 
 
 class OnchipEmulated:
-    def __init__(self, engine, net, precision, variant, workdir, extra=()):
-        src = engine.spec_source(net, precision, variant)
+    def __init__(self, engine, net, precision, variant, workdir, extra=(), env=None):
+        """env: generator knobs for this kernel (e.g. BNBP_OC_ROLES), set while its source is generated."""
+        env = env or {}
+        src = generated_source(engine, net, precision, variant, env)
         for ptx, host in PTX:                       # the three inline-PTX statements of the kernel, see onchip_emul.cpp
             assert src.count(ptx) == 1, ptx
             src = src.replace(ptx, host)
-        tag = f"{net.name}_{precision}_v{variant}"
+        tag = f"{net.name}_{precision}_v{variant}" + "".join(f"_{k}{v}" for k, v in sorted(env.items()))
         cu, so = os.path.join(workdir, tag + ".cu"), os.path.join(workdir, tag + ".so")
         with open(cu, "w") as f:
             f.write(src)
