@@ -24,7 +24,7 @@ HEADERS = [os.path.join(CSRC, "bnbp_kernels.cuh"), os.path.join(CSRC, "bnbp_swee
            os.path.join(CSRC, "bnbp_variants.h"), os.path.join(CSRC, "bnbp_jit.h"), SPEC_SRC, ONCHIP_SRC,
            os.path.join(CSRC, "bnbp_dense.h"), os.path.join(CSRC, "bnbp_dense.cuh"),
            os.path.join(CSRC, "bnbp_dense_tc.cuh"), os.path.join(CSRC, "bnbp_lw.cuh"),
-           os.path.join(os.path.dirname(HERE), "include", "bnbp.h")]
+           os.path.join(CSRC, "bnbp_logev.cuh"), os.path.join(os.path.dirname(HERE), "include", "bnbp.h")]
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 # host-only units: rebuilt when the drop-in headers they wrap change
 HOST_HEADERS = {"bnbp_netfile.cpp": [os.path.join(INCLUDE, "bayesian", "graph.hpp"),

@@ -5,6 +5,7 @@
 #include "../../include/bnbp.h"
 #include "bnbp_kernels.cuh"
 #include "bnbp_lw.cuh"
+#include "bnbp_logev.cuh"
 #include "bnbp_variants.h"
 #include "bnbp_jit.h"
 #include "bnbp_dense.h"
@@ -169,7 +170,9 @@ struct bnbp_handle {
     int rmax = 2;              // template bound actually used (2,4,8,16,32,64)
     int knet = 2;              // in-degree bound actually used (2,4,8)
     int vec = 1;
-    int tb = 128;              // cases per tile = BLOCK_THREADS * vec
+    int vec_run = 1;           // this run's VEC of the generic kernel: vec, or 1 for log-evidence in epsilon mode (a thread
+                               // of two cases rewrites a frozen case's messages while the other one runs)
+    int tb = 128;              // cases per tile = BLOCK_THREADS * vec_run
     int scratch_vals = 0;      // per-thread scratch values (x VEC)
     int64_t cpt_values = 0;
     int64_t max_resident = 0;
@@ -257,6 +260,9 @@ struct bnbp_handle {
     bool lw_ready = false;
     void* pin_counts = nullptr;         // pinned host staging of the per-case sweep counts / converged flags
     size_t pin_counts_bytes = 0;
+    DevBuf s_out_logev;                 // log-evidence of the whole batch (host-buffer call), and its pinned staging
+    double* pin_logev = nullptr;
+    size_t pin_logev_bytes = 0;
     DevBuf s_out_all;                   // whole-batch output staging (used when HBM has the room)
     cudaStream_t copy_stream = nullptr, h2d_stream = nullptr;
     std::vector<cudaEvent_t> ev_chunk;  // per chunk of the host-buffer call: uploaded, computed, copied
@@ -307,7 +313,7 @@ cudaError_t launch_sweep(const bnbp_handle* h, const SweepArgs<T>& a, dim3 grid,
                          bool check, cudaStream_t st, bool maxp = false)
 {
 #define BNBP_X(TT, V, R, K) \
-    if (h->vec == V && h->rmax == R && h->knet == K) return launch_sweep_vr<TT, V, R, K>(a, grid, smem, freeze, check, st, maxp);
+    if (h->vec_run == V && h->rmax == R && h->knet == K) return launch_sweep_vr<TT, V, R, K>(a, grid, smem, freeze, check, st, maxp);
     BNBP_SWEEP_VARIANTS(BNBP_X, T)
 #undef BNBP_X
     return cudaErrorInvalidConfiguration;
@@ -317,7 +323,7 @@ template <typename T>
 cudaError_t set_smem(const bnbp_handle* h, int bytes)
 {
 #define BNBP_X(TT, V, R, K) \
-    if (h->vec == V && h->rmax == R && h->knet == K) return set_sweep_smem<TT, V, R, K>(bytes);
+    if (h->vec_run == V && h->rmax == R && h->knet == K) return set_sweep_smem<TT, V, R, K>(bytes);
     BNBP_SWEEP_VARIANTS(BNBP_X, T)
 #undef BNBP_X
     return cudaErrorInvalidConfiguration;
@@ -491,9 +497,14 @@ int ensure_onchip(bnbp_handle* h, int idx)
 // Kernel family of one run.  Decided before the state is initialised because the tile width
 // (cases per thread) belongs to the family.  ALWAYS: failure is an error; AUTO: the generic GPU
 // kernel takes over (still CUDA: there is no CPU path).
-int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, bool soft_evidence, bool out_double)
+// logev: the run also scores each case (log_evidence_kernel), which reads the message buffers the case's last sweep
+// read.  The on-chip kernel keeps no state in HBM, the fused last sweep writes beliefs instead of the state, and the
+// split convergence test keeps sweeping retired cases: none of them is taken.
+int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, bool soft_evidence, bool out_double,
+                   bool logev = false)
 {
     h->run_spec = false;
+    h->vec_run = (logev && prm.epsilon > 0.0) ? 1 : h->vec;
     h->fuse = false;
     h->split = false;
     h->run_onchip = false;
@@ -502,7 +513,7 @@ int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, 
         // opt-in extension: the generic kernel's max flavour (one kernel per network shape class); matrix products
         // cannot take a maximum, so handles whose large CPTs sit on the dense contraction path refuse it
         if (h->TS > 0) return fail(BNBP_ERR_INVALID, "max-product: create the handle with dense_min_cpt = -1 (the dense contraction path sums)");
-        h->tb = BLOCK_THREADS * h->vec;
+        h->tb = BLOCK_THREADS * h->vec_run;
         h->last_specialised = 0;
         return BNBP_OK;
     }
@@ -516,7 +527,9 @@ int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, 
         // 357-381 M for the streaming kernels with the split convergence test (r02b vs r01fin)
         const bool plain_run = !(prm.epsilon > 0.0) && prm.damping == 0.0;
         const bool want_oc = mode > 0 || (mode == 0 && h->specialize == BNBP_SPEC_AUTO && h->oc_eligible && h->oc_auto_ok &&
-                                          !soft_evidence && n_cases >= 4096 && plain_run);
+                                          !soft_evidence && n_cases >= 4096 && plain_run && !logev);
+        if (want_oc && logev)
+            return fail(BNBP_ERR_INVALID, "onchip=ALWAYS: log-evidence reads the final messages from HBM, where the on-chip kernel keeps no state");
         if (want_oc) {
             if (!h->oc_eligible) return fail(BNBP_ERR_INVALID, "onchip=ALWAYS but the network is not eligible: " + h->oc_why);
             if (soft_evidence) return fail(BNBP_ERR_INVALID, "onchip=ALWAYS: soft evidence rows take the streaming kernels");
@@ -539,8 +552,14 @@ int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, 
         // The freeze / check variants (epsilon mode below the split threshold, damping) keep per-case state one block must
         // own, so a small batch would leave most SMs idle; the generic kernel splits its node walk in every flavour.
         const bool plain_variants = (!(prm.epsilon > 0.0) && prm.damping == 0.0) ||
-                                    (prm.epsilon > 0.0 && prm.damping == 0.0 && n_cases >= 16384 && !getenv("BNBP_NO_SPLIT"));
+                                    (prm.epsilon > 0.0 && prm.damping == 0.0 && n_cases >= 16384 && !getenv("BNBP_NO_SPLIT") && !logev);
         if (!plain_variants && n_cases < 32768) want = false;
+    }
+    if (want && logev && prm.epsilon > 0.0 && h->spec_vec != 1) {
+        // several cases per thread: a frozen case's messages are rewritten while the others run (see vec_run)
+        if (h->specialize == BNBP_SPEC_ALWAYS)
+            return fail(BNBP_ERR_INVALID, "specialize=ALWAYS: log-evidence in epsilon mode needs one case per thread (BNBP_SPEC_VEC=1)");
+        want = false;
     }
     if (want) {
         if (!h->spec_eligible_)
@@ -552,7 +571,7 @@ int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, 
         // messages are never read, so neither is moved through HBM (variants 3 and 4)
         // eps mode without damping on a batch worth it: the convergence test is a kernel of its own
         // (delta_retire_kernel) and the sweeps run as the plain variant
-        const bool split = eps_mode && prm.damping == 0.0 && n_cases >= 16384 && h->TS == 0 && !getenv("BNBP_NO_SPLIT");
+        const bool split = eps_mode && prm.damping == 0.0 && n_cases >= 16384 && h->TS == 0 && !getenv("BNBP_NO_SPLIT") && !logev;
         bool need[5] = {(plain && prm.max_sweeps != 2) || split, eps_mode && interval > 1 && prm.damping == 0.0 && !split,
                         (eps_mode && !split) || prm.damping != 0.0, plain && prm.max_sweeps >= 2, plain && prm.max_sweeps >= 2};
         bool ok = true;
@@ -564,15 +583,15 @@ int choose_kernels(bnbp_handle* h, int64_t n_cases, const bnbp_run_params& prm, 
         // fixed sweep count, hard evidence, one case per thread: K0 runs inside the first sweep and K4
         // inside the last (variants 5 and 6/7), so neither the time-0 pi/lambda nor the final ones
         // cross HBM.  Soft evidence rows do not fit a state byte: the unfused sequence handles them.
-        if (ok && need[3] && !soft_evidence && h->spec_vec == 1 && h->fuse_ok && !getenv("BNBP_NO_FUSE")) {
+        if (ok && need[3] && !soft_evidence && h->spec_vec == 1 && h->fuse_ok && !getenv("BNBP_NO_FUSE") && !logev) {
             const int vlast = (h->precision == BNBP_FP32 && out_double) ? 7 : 6;
             if (ensure_spec(h, 5) == BNBP_OK && ensure_spec(h, vlast) == BNBP_OK) h->fuse = true;
             else h->fuse_ok = false;
         }
     }
     if (!h->run_spec)        // the generic family splits the convergence test off the same way (plain sweep + delta_retire_kernel)
-        h->split = prm.epsilon > 0.0 && prm.damping == 0.0 && n_cases >= 16384 && h->TS == 0 && !getenv("BNBP_NO_SPLIT");
-    h->tb = BLOCK_THREADS * (h->run_spec ? h->spec_vec : h->vec);
+        h->split = prm.epsilon > 0.0 && prm.damping == 0.0 && n_cases >= 16384 && h->TS == 0 && !getenv("BNBP_NO_SPLIT") && !logev;
+    h->tb = BLOCK_THREADS * (h->run_spec ? h->spec_vec : h->vec_run);
     h->last_specialised = h->run_spec ? 1 : 0;
     return BNBP_OK;
 }
@@ -612,10 +631,37 @@ struct DevEvidence {       // device pointers, offsets absolute with the given b
     const int64_t* ev_val_off; const double* ev_values; int64_t ev_val_base;
 };
 
-// Runs init -> sweeps -> beliefs for n (<= cap) cases whose evidence is on the device.
+// log_evidence_kernel over the positions [0, n_pos) of an arena (arguments as belief_tiled_kernel's).  Blocks are as
+// wide as the per-thread accumulator columns allow in 96 KB of shared memory (at least one warp: r <= 128).
+template <typename T>
+int launch_logev(bnbp_handle* h, const T* pl, T* const (&msg)[2], int64_t n_pos, const int32_t* orig, int only_frozen,
+                 double* d_out_logev, int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st)
+{
+    int vals = 1;
+    for (int x = 0; x < h->N; ++x) {
+        int rj = 0;
+        for (int j = 0; j < h->nodes[x].k; ++j) rj = std::max(rj, (int)h->e_card[(size_t)h->nodes[x].e0 + j]);
+        vals = std::max(vals, h->nodes[x].card + rj);
+    }
+    const int threads = std::max(32, std::min(256, (int)(96 * 1024 / (vals * 8)) / 32 * 32));
+    const size_t smem = (size_t)threads * vals * 8;
+    if (smem > 48 * 1024)
+        CU_TRY(cudaFuncSetAttribute(log_evidence_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    log_evidence_kernel<T><<<(unsigned)((n_pos + threads - 1) / threads), threads, smem, st>>>(
+        (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
+        h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
+        d_out_logev, d_out_sweeps, d_out_conv);
+    CU_TRY(cudaGetLastError());
+    h->last_kernel_launches++;
+    return BNBP_OK;
+}
+
+// Runs init -> sweeps -> beliefs for n (<= cap) cases whose evidence is on the device.  d_out_logev: also the
+// log-evidence of each case (choose_kernels was told); d_out may then be NULL (no marginals).
 template <typename T, typename OUT>
 int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out,
-              int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps)
+              int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps,
+              double* d_out_logev = nullptr)
 {
     NvtxRange nvtx_chunk("bnbp: chunk (init, sweeps, beliefs) streaming kernels");
     const int tiles = (int)((n + h->tb - 1) / h->tb);
@@ -708,7 +754,11 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
         sa.prefetch = knob >= 0 ? knob : (h->rmax <= 4 ? 1 : 0);
     }
     T* delta = (T*)h->d_delta.p;
-    const size_t smem = (size_t)BLOCK_THREADS * (size_t)h->scratch_vals * h->vec * sizeof(T);
+    const size_t smem = (size_t)BLOCK_THREADS * (size_t)h->scratch_vals * h->vec_run * sizeof(T);
+    if (h->vec_run != h->vec && !h->run_spec && smem > 48 * 1024) {        // the handle opted in for its own VEC only
+        cudaError_t e = set_smem<T>(h, (int)smem);
+        if (e != cudaSuccess) return fail(BNBP_ERR_CUDA, std::string("shared-memory opt-in: ") + cudaGetErrorString(e));
+    }
     dim3 grid(tiles, n_chunks);
     auto regrid = [&]() {                    // after a compaction: fewer tiles, maybe more node chunks
         const int64_t tpr = (int64_t)tiles_cur * BLOCK_THREADS;
@@ -920,7 +970,7 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
                              h->d_src_pos.ensure((size_t)h->cap * 4)))
                     fits = false;
                 if (fits && split) have_total = false;           // the counts describe the old arena
-                if (fits && !split) {
+                if (fits && !split && d_out) {
                     // 1. retire the converged cases: their state is final (:135-147), write their beliefs now
                     bnbp_handle::BeliefPlan* plan = nullptr;
                     if ((rc = belief_plan(h, h->tb, (int)sizeof(OUT), &plan))) return rc;
@@ -933,6 +983,10 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
                     CU_TRY(cudaGetLastError());
                     h->last_kernel_launches++;
                 }
+                if (fits && !split && d_out_logev &&
+                    (rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 1, d_out_logev, d_out ? nullptr : d_out_sweeps,
+                                          d_out ? nullptr : d_out_conv, st)))
+                    return rc;
                 if (fits) {
                     // 2. new position -> old position (stable), 3. gather into the other arena
                     compact_scan_kernel<<<1, 1024, 0, st>>>(d_tile_cnt, d_tile_off, tiles_cur);
@@ -1002,7 +1056,7 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
             CU_TRY(cudaGetLastError());
             h->last_kernel_launches++;
         }
-    } else {
+    } else if (d_out) {
         bnbp_handle::BeliefPlan* plan = nullptr;
         int rc = belief_plan(h, h->tb, (int)sizeof(OUT), &plan);
         if (rc) return rc;
@@ -1020,6 +1074,11 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
         }
         CU_TRY(cudaGetLastError());
         h->last_kernel_launches++;
+    }
+    if (d_out_logev) {
+        const int rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 0, d_out_logev, d_out ? nullptr : d_out_sweeps,
+                                       d_out ? nullptr : d_out_conv, st);
+        if (rc) return rc;
     }
     if (planned_sweeps) *planned_sweeps = eps_mode ? -1 : (int64_t)total_sweeps * n;
     return BNBP_OK;
@@ -1135,13 +1194,15 @@ __global__ void gather_columns_kernel(const OUT* __restrict__ src, OUT* __restri
 // only those in the first place).
 template <typename T, typename OUT>
 int run_any(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out, int32_t* d_out_sweeps,
-            uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps)
+            uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps, double* d_out_logev = nullptr)
 {
     if (h->run_onchip) return run_onchip<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps);
-    if (h->q_nodes.empty()) return run_chunk<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps);
+    if (h->q_nodes.empty() || !d_out)
+        return run_chunk<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev);
     int rc = h->s_full.ensure((size_t)n * h->V * sizeof(OUT));
     if (rc) return rc;
-    if ((rc = run_chunk<T, OUT>(h, n, de, prm, (OUT*)h->s_full.p, d_out_sweeps, d_out_conv, st, planned_sweeps))) return rc;
+    if ((rc = run_chunk<T, OUT>(h, n, de, prm, (OUT*)h->s_full.p, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev)))
+        return rc;
     const int64_t total = n * h->Vout;
     if (total > 0) {
         gather_columns_kernel<OUT><<<(unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(
@@ -1771,6 +1832,7 @@ int build_layout(const bnbp_flat_network* net, const bnbp_options* opt, bnbp_han
         const int v = atoi(ev);
         if ((v == 1 || v == 2) && h->rmax <= 8) h->vec = v;
     }
+    h->vec_run = h->vec;
     h->tb = BLOCK_THREADS * h->vec;
     h->cpt_values = net->cpt_off[N];
     if (generic_smem(h) > 200 * 1024) return fail(BNBP_ERR_INVALID, "parent sets too wide for the shared-memory scratch");
@@ -1904,11 +1966,26 @@ int build_layout(const bnbp_flat_network* net, const bnbp_options* opt, bnbp_han
     return BNBP_OK;
 }
 
+// What the log-evidence calls refuse (before anything is enqueued, so the handle stays usable).
+int logev_refusal(const bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const double* out_logev)
+{
+    if (!out_logev) return fail(BNBP_ERR_INVALID, "log-evidence: out_log_evidence is NULL");
+    if (ev->ev_values)
+        return fail(BNBP_ERR_INVALID, "log-evidence takes hard evidence: soft evidence rows are not an indicator factor");
+    if (prm->semiring == BNBP_MAX_PRODUCT)
+        return fail(BNBP_ERR_INVALID, "log-evidence is a sum-product quantity: BNBP_MAX_PRODUCT is refused");
+    const bnbp_handle* l = h->members.empty() ? h : h->members[0];
+    if (l->TS > 0)
+        return fail(BNBP_ERR_INVALID, "log-evidence: the handle has dense-path nodes; create it with dense_min_cpt = -1");
+    if (prm->gather) return fail(BNBP_ERR_INVALID, "log-evidence: gather is not supported (the scores stay on this rank)");
+    return BNBP_OK;
+}
+
 // bnbp_run_batch on a group handle (bnbp_create_multi): contiguous case ranges, one host thread per device, every
 // device copies its rows straight into the caller's buffers; then the convergence summary is all-reduced over the
 // group's communicator (one grouped NCCL call from this thread).
 int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals, int32_t* out_sweeps,
-              uint8_t* out_converged)
+              uint8_t* out_converged, double* out_logev)
 {
     if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
     if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
@@ -1925,9 +2002,11 @@ int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* pr
         bnbp_evidence e = *ev;
         e.n_cases = hi[(size_t)i] - lo[(size_t)i];
         e.ev_off = ev->ev_off ? ev->ev_off + lo[(size_t)i] : nullptr;
-        rcs[(size_t)i] = bnbp_run_batch(g->members[(size_t)i], &e, prm, (char*)out_marginals + (size_t)lo[(size_t)i] * row_bytes,
-                                        out_sweeps ? out_sweeps + lo[(size_t)i] : nullptr,
-                                        out_converged ? out_converged + lo[(size_t)i] : nullptr);
+        void* const marg = out_marginals ? (char*)out_marginals + (size_t)lo[(size_t)i] * row_bytes : nullptr;
+        int32_t* const sw = out_sweeps ? out_sweeps + lo[(size_t)i] : nullptr;
+        uint8_t* const cv = out_converged ? out_converged + lo[(size_t)i] : nullptr;
+        rcs[(size_t)i] = out_logev ? bnbp_run_batch_log_evidence(g->members[(size_t)i], &e, prm, marg, sw, cv, out_logev + lo[(size_t)i])
+                                   : bnbp_run_batch(g->members[(size_t)i], &e, prm, marg, sw, cv);
         if (rcs[(size_t)i]) errs[(size_t)i] = bnbp_last_error();      // the error channel is thread-local
     };
     std::vector<std::thread> threads;
@@ -2076,7 +2155,7 @@ void bnbp_destroy(bnbp_handle* h)
                       &h->d_pl2, &h->d_msg2[0], &h->d_msg2[1], &h->d_evbits2, &h->d_orig[0], &h->d_orig[1], &h->d_src_pos, &h->d_tile_count,
                       &h->d_evst, &h->d_lw_order, &h->d_lw_par, &h->d_lw_cpt, &h->d_lw_out, &h->d_lw_wsum, &h->d_djobs, &h->d_dytab, &h->d_ddig, &h->d_cpt_t, &h->d_tscr,
                       &h->s_ev_off, &h->s_ev_node, &h->s_ev_state, &h->s_ev_val_off, &h->s_ev_values, &h->s_out[0], &h->s_out[1], &h->s_out_all,
-                      &h->s_out_sweeps, &h->s_out_conv})
+                      &h->s_out_sweeps, &h->s_out_conv, &h->s_out_logev})
         b->release();
     for (auto& kv : h->belief_plans) kv.second.groups.release();
     for (cudaEvent_t e : h->ev_chunk) cudaEventDestroy(e);
@@ -2092,6 +2171,7 @@ void bnbp_destroy(bnbp_handle* h)
     }
     if (h->pinned_poll) cudaFreeHost(h->pinned_poll);
     if (h->pin_counts) cudaFreeHost(h->pin_counts);
+    if (h->pin_logev) cudaFreeHost(h->pin_logev);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
 }
@@ -2198,13 +2278,13 @@ int bnbp_spec_source(const bnbp_flat_network* net, const bnbp_options* opt, int3
     return BNBP_OK;
 }
 
-int bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
-                          int32_t* out_sweeps, uint8_t* out_converged, void* stream)
+static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
+                            int32_t* out_sweeps, uint8_t* out_converged, double* out_logev, void* stream)
 {
-    if (!h || !ev || !out_marginals) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device: NULL argument");
     NvtxRange nvtx_call("bnbp_run_batch_device");
     int rc = validate_params(prm);
     if (rc) return rc;
+    if (out_logev && (rc = logev_refusal(h, ev, prm, out_logev))) return rc;
     if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
     if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
     CU_TRY(cudaSetDevice(h->device));
@@ -2217,7 +2297,7 @@ int bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     if (ev->n_cases == 0) return BNBP_OK;
     if (!h->members.empty()) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device: a group handle takes host buffers (bnbp_run_batch); the device path belongs to one device");
     if ((rc = set_query(h, *prm))) return rc;
-    if ((rc = choose_kernels(h, ev->n_cases, *prm, ev->ev_values != nullptr, h->precision != BNBP_FP32))) return rc;
+    if ((rc = choose_kernels(h, ev->n_cases, *prm, ev->ev_values != nullptr, h->precision != BNBP_FP32, out_logev != nullptr))) return rc;
     if (!h->run_onchip && (rc = ensure_state(h, ev->n_cases))) return rc;
     // a flag left by an earlier (unchecked, asynchronous) run must not fail this one
     CU_TRY(cudaMemsetAsync(reinterpret_cast<int32_t*>(h->d_misc.p) + 1, 0, 4, st));
@@ -2252,13 +2332,14 @@ int bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
         const int64_t n = std::min<int64_t>(step_cases, ev->n_cases - c0);
         DevEvidence de{ev->ev_off + c0, 0, ev->ev_node, ev->ev_state, ev->ev_val_off, ev->ev_values, 0};
         int64_t planned = 0;
-        char* const dst = mine + (size_t)c0 * row_bytes;
+        char* const dst = out_marginals ? mine + (size_t)c0 * row_bytes : nullptr;
+        double* const lev = out_logev ? out_logev + c0 : nullptr;
         if (h->precision == BNBP_FP32)
             rc = run_any<float, float>(h, n, de, *prm, (float*)dst, out_sweeps ? out_sweeps + c0 : nullptr,
-                                       out_converged ? out_converged + c0 : nullptr, st, &planned);
+                                       out_converged ? out_converged + c0 : nullptr, st, &planned, lev);
         else
             rc = run_any<double, double>(h, n, de, *prm, (double*)dst, out_sweeps ? out_sweeps + c0 : nullptr,
-                                         out_converged ? out_converged + c0 : nullptr, st, &planned);
+                                         out_converged ? out_converged + c0 : nullptr, st, &planned, lev);
         if (rc) return rc;
         if (planned < 0) exact = false; else h->last_case_sweeps += planned;
         if (exchange) {
@@ -2298,6 +2379,20 @@ int bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     return BNBP_OK;
 }
 
+int bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
+                          int32_t* out_sweeps, uint8_t* out_converged, void* stream)
+{
+    if (!h || !ev || !out_marginals) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device: NULL argument");
+    return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, nullptr, stream);
+}
+
+int bnbp_run_batch_device_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
+                                       int32_t* out_sweeps, uint8_t* out_converged, double* out_log_evidence, void* stream)
+{
+    if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device_log_evidence: NULL argument");
+    return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, stream);
+}
+
 int bnbp_check_errors(bnbp_handle* h, void* stream)
 {
     if (!h) return fail(BNBP_ERR_INVALID, "bnbp_check_errors: NULL handle");
@@ -2306,15 +2401,15 @@ int bnbp_check_errors(bnbp_handle* h, void* stream)
     return check_error_flag(h, stream ? (cudaStream_t)stream : h->stream);
 }
 
-int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals_v,
-                   int32_t* out_sweeps, uint8_t* out_converged)
+static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals_v,
+                          int32_t* out_sweeps, uint8_t* out_converged, double* out_logev)
 {
-    if (!h || !ev || !out_marginals_v) return fail(BNBP_ERR_INVALID, "bnbp_run_batch: NULL argument");
     const auto t_entry = std::chrono::steady_clock::now();
     NvtxRange nvtx_call("bnbp_run_batch (host buffers: H2D evidence | kernels | D2H marginals, pipelined by chunk)");
     int rc = validate_params(prm);
     if (rc) return rc;
-    if (!h->members.empty()) return run_group(h, ev, prm, out_marginals_v, out_sweeps, out_converged);
+    if (out_logev && (rc = logev_refusal(h, ev, prm, out_logev))) return rc;
+    if (!h->members.empty()) return run_group(h, ev, prm, out_marginals_v, out_sweeps, out_converged, out_logev);
     const bool out_f32 = prm->out_precision == BNBP_OUT_FP32;
     if (out_f32 && h->precision != BNBP_FP32)
         return fail(BNBP_ERR_INVALID, "out_precision FP32 needs an fp32 handle (an fp64 handle returns the reference's doubles)");
@@ -2340,7 +2435,7 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
     if (ev->n_cases == 0) return BNBP_OK;
     h->reserve_sms = 0;
     if ((rc = set_query(h, *prm))) return rc;
-    if ((rc = choose_kernels(h, ev->n_cases, *prm, soft, !out_f32))) return rc;
+    if ((rc = choose_kernels(h, ev->n_cases, *prm, soft, !out_f32, out_logev != nullptr))) return rc;
     if ((rc = measure_rates(h))) return rc;
     // Chunk pipeline on three streams: evidence of chunk i+1 goes up (h2d_stream) and the marginals of
     // chunk i-1 come down (copy_stream) while init/sweeps/beliefs of chunk i run.  Marginals are 8*V
@@ -2382,6 +2477,7 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
     // else a ring of two chunk-sized slots.
     const size_t row_bytes = (size_t)h->Vout * out_elem;
     bool whole = (size_t)ev->n_cases * row_bytes <= h->s_out_all.bytes;
+    if (!out_marginals) whole = true;                     // no marginals asked (log-evidence only): nothing to stage
     if (!whole && !getenv("BNBP_STAGING_RING")) {
         size_t free_b = 0, total_b = 0;
         CU_TRY(cudaMemGetInfo(&free_b, &total_b));
@@ -2407,6 +2503,16 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
     }
     int32_t* const pin_sweeps = (int32_t*)h->pin_counts;
     uint8_t* const pin_conv = (uint8_t*)h->pin_counts + (size_t)ev->n_cases * 4;
+    if (out_logev) {
+        if ((rc = h->s_out_logev.ensure((size_t)ev->n_cases * 8))) return rc;
+        if (h->pin_logev_bytes < (size_t)ev->n_cases * 8) {
+            if (h->pin_logev) cudaFreeHost(h->pin_logev);
+            h->pin_logev = nullptr;
+            h->pin_logev_bytes = 0;
+            CU_TRY(cudaMallocHost((void**)&h->pin_logev, (size_t)ev->n_cases * 8));
+            h->pin_logev_bytes = (size_t)ev->n_cases * 8;
+        }
+    }
     // evidence staging for the whole batch (absolute offsets, like bnbp_run_batch_device)
     if ((rc = h->s_ev_off.ensure((size_t)(ev->n_cases + 1) * 8))) return rc;
     if ((rc = h->s_ev_node.ensure(std::max<size_t>(16, (size_t)nnz * 4)))) return rc;
@@ -2494,23 +2600,26 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
         CU_TRY(cudaEventRecord(e_up, hs));
         nvtx_h2d.reset();
         CU_TRY(cudaStreamWaitEvent(st, e_up, 0));
-        char* slot = whole ? (char*)h->s_out_all.p + (size_t)c0 * row_bytes : (char*)h->s_out[idx & 1].p;
+        char* slot = !out_marginals ? nullptr : whole ? (char*)h->s_out_all.p + (size_t)c0 * row_bytes : (char*)h->s_out[idx & 1].p;
+        double* const lev = out_logev ? (double*)h->s_out_logev.p + c0 : nullptr;
         if (!whole && idx >= 2) CU_TRY(cudaStreamWaitEvent(st, h->ev_chunk[3 * (idx - 2) + 2], 0));   // ring slot is free again
         stamp("enqueue chunk", idx);
         mark(st);
         if (h->precision == BNBP_FP32 && out_f32)
-            rc = run_any<float, float>(h, n, de, *prm, (float*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr);
+            rc = run_any<float, float>(h, n, de, *prm, (float*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev);
         else if (h->precision == BNBP_FP32)
-            rc = run_any<float, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr);
+            rc = run_any<float, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev);
         else
-            rc = run_any<double, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr);
+            rc = run_any<double, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev);
         if (rc) return rc;
         mark(st);
         CU_TRY(cudaEventRecord(e_done, st));
         CU_TRY(cudaStreamWaitEvent(cs, e_done, 0));
         mark(cs);
         NvtxRange nvtx_d2h("bnbp: enqueue D2H marginals of a chunk");
-        CU_TRY(cudaMemcpyAsync(out_marginals + (size_t)c0 * row_bytes, slot, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, cs));
+        if (out_marginals)
+            CU_TRY(cudaMemcpyAsync(out_marginals + (size_t)c0 * row_bytes, slot, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, cs));
+        if (out_logev) CU_TRY(cudaMemcpyAsync(h->pin_logev + c0, lev, (size_t)n * 8, cudaMemcpyDeviceToHost, cs));
         mark(cs);
         // per-case counts: into the library's pinned staging (the caller's arrays are usually pageable, and
         // a pageable D2H would block this thread until the chunk is done)
@@ -2545,6 +2654,7 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
     for (cudaEvent_t e : tev) cudaEventDestroy(e);
     if (out_sweeps) memcpy(out_sweeps, pin_sweeps, (size_t)ev->n_cases * 4);
     if (out_converged) memcpy(out_converged, pin_conv, (size_t)ev->n_cases);
+    if (out_logev) memcpy(out_logev, h->pin_logev, (size_t)ev->n_cases * 8);
     if (!(prm->epsilon > 0.0)) {
         h->last_case_sweeps = ev->n_cases * (int64_t)prm->max_sweeps;     // fixed count: every case ran them all
     } else if (out_sweeps) {
@@ -2556,6 +2666,20 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
     }
     h->last_host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_entry).count();
     return BNBP_OK;
+}
+
+int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
+                   int32_t* out_sweeps, uint8_t* out_converged)
+{
+    if (!h || !ev || !out_marginals) return fail(BNBP_ERR_INVALID, "bnbp_run_batch: NULL argument");
+    return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, nullptr);
+}
+
+int bnbp_run_batch_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
+                                int32_t* out_sweeps, uint8_t* out_converged, double* out_log_evidence)
+{
+    if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_log_evidence: NULL argument");
+    return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence);
 }
 
 int bnbp_lw_run_batch(bnbp_handle* h, const bnbp_evidence* ev, int64_t n_samples, uint64_t seed, double* out_marginals,

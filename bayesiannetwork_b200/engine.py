@@ -67,6 +67,7 @@ class BPResult:
     marginals: np.ndarray      # [n_cases, sum r_X] (float64 on the host path)
     sweeps: np.ndarray         # [n_cases] int32
     converged: np.ndarray      # [n_cases] uint8
+    log_evidence: Optional[np.ndarray] = None   # [n_cases] float64, Bethe estimate of ln P(e) (log_evidence=True)
 
     def node(self, net: FlatNetwork, x: int) -> np.ndarray:
         off = net.belief_off
@@ -124,10 +125,17 @@ class BeliefPropagation:
                  max_sweeps: int = 0, damping: float = 0.0, check_interval: int = 1,
                  out: Optional[np.ndarray] = None, out_sweeps: Optional[np.ndarray] = None,
                  out_converged: Optional[np.ndarray] = None, query_nodes: Optional[Sequence[int]] = None,
-                 out_dtype=np.float64, semiring: str = "sum") -> BPResult:
+                 out_dtype=np.float64, semiring: str = "sum", log_evidence: bool = False,
+                 marginals: bool = True) -> BPResult:
         """``query_nodes``: only these nodes' marginals are returned (columns in the given order);
         ``out_dtype=np.float32`` (fp32 handles): float marginals, half the device-to-host copy;
-        ``semiring="max"``: max-product (max-marginals) instead of the reference's sum-product."""
+        ``semiring="max"``: max-product (max-marginals) instead of the reference's sum-product;
+        ``log_evidence=True``: also each case's Bethe estimate of ln P(e) (``bnbp_run_batch_log_evidence``; exact on
+        polytrees run to convergence; hard evidence only) in ``BPResult.log_evidence``;
+        ``marginals=False`` (with ``log_evidence``): no marginals are computed into or copied to the host, the result's
+        marginals are an (n, 0) array."""
+        if not marginals and not log_evidence:
+            raise ValueError("marginals=False needs log_evidence=True (the call would return nothing)")
         if evidence is None:
             evidence = EvidenceBatch.empty(1)   # operator()(epsilon) by-pass (:24-28)
         ev = evidence
@@ -137,9 +145,12 @@ class BeliefPropagation:
             raise BnbpError(1, "query node id out of range")
         V = self.net.belief_values if q is None or q.size == 0 else int(self.net.card[q].sum())
         out_dtype = np.dtype(out_dtype)
-        if out is None:
+        if not marginals:
+            out = np.empty((n, 0), dtype=out_dtype)
+        elif out is None:
             out = np.empty((n, V), dtype=out_dtype)
-        assert out.dtype == out_dtype and out.size == n * V and out.flags.c_contiguous
+        if marginals:
+            assert out.dtype == out_dtype and out.size == n * V and out.flags.c_contiguous
         # caller-owned result buffers (all three optional) keep a hot loop free of multi-megabyte
         # allocations: every fresh array is an mmap + page faults + munmap on the calling thread
         sweeps = np.empty(n, dtype=np.int32) if out_sweeps is None else out_sweeps
@@ -153,6 +164,12 @@ class BeliefPropagation:
         prm = _capi.RunParamsC(float(epsilon), int(max_sweeps), float(damping), int(check_interval),
                                2 if out_dtype == np.float32 else 0, 0, 0 if q is None else int(q.size), _vp(q),
                                {"sum": 0, "max": 1}[semiring])
+        if log_evidence:
+            logev = np.empty(n, dtype=np.float64)
+            _capi.check(self._lib.bnbp_run_batch_log_evidence(self._h, C.byref(evc), C.byref(prm),
+                                                              _vp(out) if marginals else None, _vp(sweeps), _vp(conv),
+                                                              _vp(logev)))
+            return BPResult(out.reshape(n, V if marginals else 0), sweeps, conv, logev)
         _capi.check(self._lib.bnbp_run_batch(self._h, C.byref(evc), C.byref(prm), _vp(out), _vp(sweeps), _vp(conv)))
         return BPResult(out.reshape(n, V), sweeps, conv)
 
@@ -160,10 +177,12 @@ class BeliefPropagation:
     def run_device(self, n_cases: int, ev_off, ev_node, ev_state, out, *, ev_val_off=None, ev_values=None,
                    epsilon: float = 0.0, max_sweeps: int = 20, damping: float = 0.0, check_interval: int = 1,
                    out_sweeps=None, out_converged=None, stream: int = 0, gather: bool = False,
-                   query_nodes: Optional[Sequence[int]] = None) -> None:
+                   query_nodes: Optional[Sequence[int]] = None, out_log_evidence=None) -> None:
         """All tensor arguments are CUDA tensors (int64 / int32 / float64 offsets and values as in
         ``bnbp_evidence``); ``out`` has the handle's precision, shape [n_cases, sum r_X].
-        Work is enqueued on ``stream`` (a raw cudaStream_t, e.g. torch.cuda.current_stream().cuda_stream)."""
+        Work is enqueued on ``stream`` (a raw cudaStream_t, e.g. torch.cuda.current_stream().cuda_stream).
+        ``out_log_evidence``: a float64 CUDA tensor [n_cases] that receives each case's Bethe log-evidence
+        (``bnbp_run_batch_device_log_evidence``); ``out`` may then be None (no marginals)."""
         def dp(t):
             return None if t is None else int(t.data_ptr())
         evc = _capi.EvidenceC(int(n_cases), dp(ev_off), dp(ev_node), dp(ev_state), dp(ev_val_off), dp(ev_values))
@@ -172,8 +191,15 @@ class BeliefPropagation:
         # place and exchanged over NCCL inside the call
         prm = _capi.RunParamsC(float(epsilon), int(max_sweeps), float(damping), int(check_interval), 0,
                                1 if gather else 0, 0 if q is None else int(q.size), _vp(q))
+        st = C.c_void_p(stream) if stream else None
+        if out_log_evidence is not None:
+            assert out_log_evidence.dtype.itemsize == 8 and out_log_evidence.is_floating_point() and out_log_evidence.is_cuda
+            assert out_log_evidence.numel() == int(n_cases) and out_log_evidence.is_contiguous()
+            _capi.check(self._lib.bnbp_run_batch_device_log_evidence(self._h, C.byref(evc), C.byref(prm), dp(out), dp(out_sweeps),
+                                                                     dp(out_converged), dp(out_log_evidence), st))
+            return
         _capi.check(self._lib.bnbp_run_batch_device(self._h, C.byref(evc), C.byref(prm), dp(out), dp(out_sweeps),
-                                                    dp(out_converged), C.c_void_p(stream) if stream else None))
+                                                    dp(out_converged), st))
 
     # ---- several processes, one GPU each: the communicator lives in the library (SURVEY 8e) --------
     @staticmethod

@@ -115,6 +115,7 @@ public:
         // run_flat only -- what leaves the device (the map-returning overloads always return every vertex in double):
         std::vector<vertex_type> query;   // non-empty: only these vertices' marginals, in this order
         bool float_marginals = false;     // fp32 handles: marginals_f32 is filled instead of marginals (half the copy)
+        bool log_evidence = false;        // flat_result::log_evidence: each case's Bethe estimate of ln P(e) (hard evidence)
     };
 
     struct flat_result {
@@ -126,6 +127,7 @@ public:
         pinned_buffer<float> marginals_f32;        // [n_cases][values_per_case] (only if float_marginals)
         pinned_buffer<std::int32_t> sweeps;        // sweeps executed per case
         pinned_buffer<std::uint8_t> converged;     // 1 if the case met delta < epsilon
+        std::vector<double> log_evidence;          // options::log_evidence: per case (bnbp_run_batch_log_evidence), else empty
         bnbp_summary summary = bnbp_summary();     // totals over all devices (devices.size() > 1: all-reduced over NCCL)
     };
 
@@ -333,8 +335,16 @@ private:
         prm.semiring = opt.semiring;
         prm.n_query = static_cast<std::int32_t>(query.size());
         prm.query_nodes = query.empty() ? nullptr : query.data();
-        if (bnbp_run_batch(handle_, &ev, &prm, dst, out.sweeps.data(), out.converged.data()) != BNBP_OK)
-            throw std::runtime_error(last_error("bnbp_run_batch"));
+        if (opt.log_evidence) {
+            out.log_evidence.resize(out.n_cases);
+            if (bnbp_run_batch_log_evidence(handle_, &ev, &prm, dst, out.sweeps.data(), out.converged.data(),
+                                            out.log_evidence.data()) != BNBP_OK)
+                throw std::runtime_error(last_error("bnbp_run_batch_log_evidence"));
+        } else {
+            out.log_evidence.clear();
+            if (bnbp_run_batch(handle_, &ev, &prm, dst, out.sweeps.data(), out.converged.data()) != BNBP_OK)
+                throw std::runtime_error(last_error("bnbp_run_batch"));
+        }
         if (!opt.devices.empty()) bnbp_get_summary(handle_, &out.summary);
     }
 
@@ -343,6 +353,7 @@ private:
     {
         opt.query.clear();
         opt.float_marginals = false;
+        opt.log_evidence = false;
         return opt;
     }
 

@@ -18,6 +18,7 @@
  *                         the reference runs one evidence set on one core)
  *   bnbp_host_alloc/free  (new: page-locked result buffers for bnbp_run_batch)
  *   bnbp_check_errors  (evidence validation of the asynchronous device-path call; no reference counterpart)
+ *   bnbp_run_batch_log_evidence / bnbp_run_batch_device_log_evidence  (new: per-case Bethe log-evidence)
  *   bnbp_destroy       <- belief_propagation::~belief_propagation()   :21
  *   bnbp_last_error    <- (the reference has no error channel; UB / NaN / endless loop)
  *   bnbp_refresh_cpt   <- the reference reads vertex_t::cpt at call time (graph.hpp:157-161), so
@@ -271,6 +272,27 @@ int  bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_r
  * when it starts, so an unchecked error never fails a later call.  (The reference has no error channel:
  * evidence on a vertex outside the graph is silently ignored, belief_propagation.hpp:69-73.) */
 int  bnbp_check_errors(bnbp_handle* h, void* stream);
+
+/* Log-evidence (no reference counterpart): bnbp_run_batch / bnbp_run_batch_device that also return, per case,
+ * the Bethe estimate log Z_B of ln P(e) from the state the run ends with -- exactly ln P(e) on a polytree run to
+ * convergence, BP's standard approximation of it on a loopy network.  With the rows lambda_X of the final state and
+ * the pi-messages pm_j the case's last sweep read (the committed messages of the sweep before, damped if damping is
+ * on), per node X with parents U_j, m_X children and CPT P(x|u):
+ *   Z_X = sum_{x,u} P(x|u) lambda_X(x) prod_j pm_j(u_j),  b_X = that product / Z_X,
+ *   log Z_B = sum_X [ ln Z_X - sum_x b_X(x) ln lambda_X(x) - sum_j sum_u b_X(u_j=u) ln pm_j(u) + m_X sum_x b_X(x) ln b_X(x) ]
+ * A term of weight 0 contributes 0; a NaN Z_X makes the case NaN, else a zero Z_X makes it -inf (evidence impossible
+ * given the messages).  fp64 sums in both precisions.  out_log_evidence [n_cases] doubles (host / device memory as
+ * the call's other outputs).  out_marginals may be NULL: then no marginals are written or copied.  Group handles
+ * slice it like out_sweeps.  The run takes the streaming kernels (not the on-chip kernel, the fused first / last
+ * sweeps or the split convergence test: AUTO steps around them, onchip = ALWAYS is refused).  BNBP_ERR_INVALID with
+ * the reason for soft evidence, BNBP_MAX_PRODUCT, handles with dense-path nodes (create with dense_min_cpt = -1)
+ * and gather; the handle stays usable. */
+int  bnbp_run_batch_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
+                                 void* out_marginals, int32_t* out_sweeps, uint8_t* out_converged,
+                                 double* out_log_evidence);
+int  bnbp_run_batch_device_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
+                                        void* out_marginals, int32_t* out_sweeps, uint8_t* out_converged,
+                                        double* out_log_evidence, void* stream);
 
 /* Likelihood weighting for a batch of HARD-evidence cases (SURVEY 8 f2): the independent statistical
  * check of BP marginals on loopy networks.  Replaces likelihood_weighting::operator()(evidence_list,
