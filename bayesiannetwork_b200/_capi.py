@@ -69,6 +69,7 @@ EXPORTS = ["bnbp_device_count", "bnbp_last_error", "bnbp_create", "bnbp_destroy"
            "bnbp_run_batch_device", "bnbp_check_errors", "bnbp_lw_run_batch", "bnbp_estimate_cpt", "bnbp_get_stats", "bnbp_refresh_cpt", "bnbp_precompile", "bnbp_spec_source",
            "bnbp_host_alloc", "bnbp_host_free", "bnbp_create_multi", "bnbp_get_summary", "bnbp_comm_unique_id",
            "bnbp_comm_init", "bnbp_comm_summary", "bnbp_run_batch_log_evidence", "bnbp_run_batch_device_log_evidence",
+           "bnbp_run_batch_expected_counts", "bnbp_run_batch_device_expected_counts",
            "bnbp_netfile_parse", "bnbp_netfile_load", "bnbp_netfile_network", "bnbp_netfile_name",
            "bnbp_netfile_node_name", "bnbp_netfile_state_name", "bnbp_netfile_free"]
 
@@ -106,6 +107,13 @@ def load():
     lib.bnbp_run_batch_device_log_evidence.restype = C.c_int
     lib.bnbp_run_batch_device_log_evidence.argtypes = [C.c_void_p, C.POINTER(EvidenceC), C.POINTER(RunParamsC),
                                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.bnbp_run_batch_expected_counts.restype = C.c_int
+    lib.bnbp_run_batch_expected_counts.argtypes = [C.c_void_p, C.POINTER(EvidenceC), C.POINTER(RunParamsC), C.c_void_p,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.bnbp_run_batch_device_expected_counts.restype = C.c_int
+    lib.bnbp_run_batch_device_expected_counts.argtypes = [C.c_void_p, C.POINTER(EvidenceC), C.POINTER(RunParamsC),
+                                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                          C.c_void_p, C.c_void_p]
     lib.bnbp_host_alloc.restype = C.c_void_p
     lib.bnbp_host_alloc.argtypes = [C.c_size_t]
     lib.bnbp_host_free.restype = None

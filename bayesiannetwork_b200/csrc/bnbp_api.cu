@@ -263,6 +263,8 @@ struct bnbp_handle {
     DevBuf s_out_logev;                 // log-evidence of the whole batch (host-buffer call), and its pinned staging
     double* pin_logev = nullptr;
     size_t pin_logev_bytes = 0;
+    DevBuf s_counts, s_weights;         // expected-counts call (host buffers): the call's zeroed count arena, the weights
+    double* pin_cnt = nullptr;          // pinned staging of the count arena (cpt_values doubles)
     DevBuf s_out_all;                   // whole-batch output staging (used when HBM has the room)
     cudaStream_t copy_stream = nullptr, h2d_stream = nullptr;
     std::vector<cudaEvent_t> ev_chunk;  // per chunk of the host-buffer call: uploaded, computed, copied
@@ -633,9 +635,12 @@ struct DevEvidence {       // device pointers, offsets absolute with the given b
 
 // log_evidence_kernel over the positions [0, n_pos) of an arena (arguments as belief_tiled_kernel's).  Blocks are as
 // wide as the per-thread accumulator columns allow in 96 KB of shared memory (at least one warp: r <= 128).
+// d_counts: the kernel's count pass also adds each scored case's family posteriors (weights d_weights, NULL = 1) into
+// it; d_out_logev may then be NULL.
 template <typename T>
 int launch_logev(bnbp_handle* h, const T* pl, T* const (&msg)[2], int64_t n_pos, const int32_t* orig, int only_frozen,
-                 double* d_out_logev, int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st)
+                 double* d_out_logev, int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st,
+                 double* d_counts = nullptr, const double* d_weights = nullptr)
 {
     int vals = 1;
     for (int x = 0; x < h->N; ++x) {
@@ -643,26 +648,40 @@ int launch_logev(bnbp_handle* h, const T* pl, T* const (&msg)[2], int64_t n_pos,
         for (int j = 0; j < h->nodes[x].k; ++j) rj = std::max(rj, (int)h->e_card[(size_t)h->nodes[x].e0 + j]);
         vals = std::max(vals, h->nodes[x].card + rj);
     }
+    if (d_counts) vals += 1;                                // + one reduction slot per thread (32 entries per warp)
     const int threads = std::max(32, std::min(256, (int)(96 * 1024 / (vals * 8)) / 32 * 32));
     const size_t smem = (size_t)threads * vals * 8;
-    if (smem > 48 * 1024)
-        CU_TRY(cudaFuncSetAttribute(log_evidence_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    log_evidence_kernel<T><<<(unsigned)((n_pos + threads - 1) / threads), threads, smem, st>>>(
-        (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
-        h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
-        d_out_logev, d_out_sweeps, d_out_conv);
+    const unsigned blocks = (unsigned)((n_pos + threads - 1) / threads);
+    if (d_counts) {
+        if (smem > 48 * 1024)
+            CU_TRY(cudaFuncSetAttribute(log_evidence_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        log_evidence_kernel<T, true><<<blocks, threads, smem, st>>>(
+            (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
+            h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
+            d_out_logev, d_out_sweeps, d_out_conv, d_weights, d_counts);
+    } else {
+        if (smem > 48 * 1024)
+            CU_TRY(cudaFuncSetAttribute(log_evidence_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        log_evidence_kernel<T, false><<<blocks, threads, smem, st>>>(
+            (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
+            h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
+            d_out_logev, d_out_sweeps, d_out_conv, nullptr, nullptr);
+    }
     CU_TRY(cudaGetLastError());
     h->last_kernel_launches++;
     return BNBP_OK;
 }
 
 // Runs init -> sweeps -> beliefs for n (<= cap) cases whose evidence is on the device.  d_out_logev: also the
-// log-evidence of each case (choose_kernels was told); d_out may then be NULL (no marginals).
+// log-evidence of each case (choose_kernels was told); d_out may then be NULL (no marginals).  d_counts: the same
+// scoring launches also add the expected family counts into it (weights d_weights of this chunk's cases, NULL = 1);
+// d_out_logev may then be NULL.
 template <typename T, typename OUT>
 int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out,
               int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps,
-              double* d_out_logev = nullptr)
+              double* d_out_logev = nullptr, double* d_counts = nullptr, const double* d_weights = nullptr)
 {
+    const bool scored = d_out_logev || d_counts;
     NvtxRange nvtx_chunk("bnbp: chunk (init, sweeps, beliefs) streaming kernels");
     const int tiles = (int)((n + h->tb - 1) / h->tb);
     int32_t* d_last_active = reinterpret_cast<int32_t*>(h->d_misc.p);
@@ -983,9 +1002,9 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
                     CU_TRY(cudaGetLastError());
                     h->last_kernel_launches++;
                 }
-                if (fits && !split && d_out_logev &&
+                if (fits && !split && scored &&
                     (rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 1, d_out_logev, d_out ? nullptr : d_out_sweeps,
-                                          d_out ? nullptr : d_out_conv, st)))
+                                          d_out ? nullptr : d_out_conv, st, d_counts, d_weights)))
                     return rc;
                 if (fits) {
                     // 2. new position -> old position (stable), 3. gather into the other arena
@@ -1075,9 +1094,9 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
         CU_TRY(cudaGetLastError());
         h->last_kernel_launches++;
     }
-    if (d_out_logev) {
+    if (scored) {
         const int rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 0, d_out_logev, d_out ? nullptr : d_out_sweeps,
-                                       d_out ? nullptr : d_out_conv, st);
+                                       d_out ? nullptr : d_out_conv, st, d_counts, d_weights);
         if (rc) return rc;
     }
     if (planned_sweeps) *planned_sweeps = eps_mode ? -1 : (int64_t)total_sweeps * n;
@@ -1194,14 +1213,17 @@ __global__ void gather_columns_kernel(const OUT* __restrict__ src, OUT* __restri
 // only those in the first place).
 template <typename T, typename OUT>
 int run_any(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out, int32_t* d_out_sweeps,
-            uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps, double* d_out_logev = nullptr)
+            uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps, double* d_out_logev = nullptr,
+            double* d_counts = nullptr, const double* d_weights = nullptr)
 {
     if (h->run_onchip) return run_onchip<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps);
     if (h->q_nodes.empty() || !d_out)
-        return run_chunk<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev);
+        return run_chunk<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev,
+                                 d_counts, d_weights);
     int rc = h->s_full.ensure((size_t)n * h->V * sizeof(OUT));
     if (rc) return rc;
-    if ((rc = run_chunk<T, OUT>(h, n, de, prm, (OUT*)h->s_full.p, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev)))
+    if ((rc = run_chunk<T, OUT>(h, n, de, prm, (OUT*)h->s_full.p, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev,
+                                d_counts, d_weights)))
         return rc;
     const int64_t total = n * h->Vout;
     if (total > 0) {
@@ -1966,26 +1988,35 @@ int build_layout(const bnbp_flat_network* net, const bnbp_options* opt, bnbp_han
     return BNBP_OK;
 }
 
-// What the log-evidence calls refuse (before anything is enqueued, so the handle stays usable).
-int logev_refusal(const bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const double* out_logev)
+// What the log-evidence and expected-counts calls refuse (before anything is enqueued, so the handle stays usable).
+// counts_call: the expected-counts call, whose counts array must be given and whose out_log_evidence may be NULL.
+int logev_refusal(const bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const double* out_logev,
+                  bool counts_call = false, const double* counts = nullptr)
 {
-    if (!out_logev) return fail(BNBP_ERR_INVALID, "log-evidence: out_log_evidence is NULL");
+    if (counts_call && !counts) return fail(BNBP_ERR_INVALID, "expected counts: counts is NULL");
+    if (!counts_call && !out_logev) return fail(BNBP_ERR_INVALID, "log-evidence: out_log_evidence is NULL");
+    const std::string what = counts_call ? "expected counts" : "log-evidence";
     if (ev->ev_values)
-        return fail(BNBP_ERR_INVALID, "log-evidence takes hard evidence: soft evidence rows are not an indicator factor");
+        return fail(BNBP_ERR_INVALID, what + (counts_call ? " take" : " takes") +
+                                          " hard evidence: soft evidence rows are not an indicator factor");
     if (prm->semiring == BNBP_MAX_PRODUCT)
-        return fail(BNBP_ERR_INVALID, "log-evidence is a sum-product quantity: BNBP_MAX_PRODUCT is refused");
+        return fail(BNBP_ERR_INVALID, what + (counts_call ? " are" : " is") + " a sum-product quantity: BNBP_MAX_PRODUCT is refused");
     const bnbp_handle* l = h->members.empty() ? h : h->members[0];
     if (l->TS > 0)
-        return fail(BNBP_ERR_INVALID, "log-evidence: the handle has dense-path nodes; create it with dense_min_cpt = -1");
-    if (prm->gather) return fail(BNBP_ERR_INVALID, "log-evidence: gather is not supported (the scores stay on this rank)");
+        return fail(BNBP_ERR_INVALID, what + ": the handle has dense-path nodes; create it with dense_min_cpt = -1");
+    if (prm->gather)
+        return fail(BNBP_ERR_INVALID, what + (counts_call ? ": gather is not supported (the counts stay on this rank)"
+                                                          : ": gather is not supported (the scores stay on this rank)"));
     return BNBP_OK;
 }
 
 // bnbp_run_batch on a group handle (bnbp_create_multi): contiguous case ranges, one host thread per device, every
 // device copies its rows straight into the caller's buffers; then the convergence summary is all-reduced over the
 // group's communicator (one grouped NCCL call from this thread).
+// counts (expected-counts call): every member adds into its own zeroed host buffer; the buffers are summed in member
+// order and the sum is added into counts.
 int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals, int32_t* out_sweeps,
-              uint8_t* out_converged, double* out_logev)
+              uint8_t* out_converged, double* out_logev, double* counts = nullptr, const double* weights = nullptr)
 {
     if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
     if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
@@ -1998,6 +2029,7 @@ int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* pr
     std::vector<std::string> errs((size_t)G);
     std::vector<int64_t> lo((size_t)G), hi((size_t)G);
     for (int i = 0; i < G; ++i) shard_range(ev->n_cases, i, G, &lo[(size_t)i], &hi[(size_t)i]);
+    std::vector<std::vector<double>> part(counts ? (size_t)G : 0, std::vector<double>((size_t)g->members[0]->cpt_values, 0.0));
     auto work = [&](int i) {
         bnbp_evidence e = *ev;
         e.n_cases = hi[(size_t)i] - lo[(size_t)i];
@@ -2005,8 +2037,13 @@ int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* pr
         void* const marg = out_marginals ? (char*)out_marginals + (size_t)lo[(size_t)i] * row_bytes : nullptr;
         int32_t* const sw = out_sweeps ? out_sweeps + lo[(size_t)i] : nullptr;
         uint8_t* const cv = out_converged ? out_converged + lo[(size_t)i] : nullptr;
-        rcs[(size_t)i] = out_logev ? bnbp_run_batch_log_evidence(g->members[(size_t)i], &e, prm, marg, sw, cv, out_logev + lo[(size_t)i])
-                                   : bnbp_run_batch(g->members[(size_t)i], &e, prm, marg, sw, cv);
+        double* const lev = out_logev ? out_logev + lo[(size_t)i] : nullptr;
+        if (counts)
+            rcs[(size_t)i] = bnbp_run_batch_expected_counts(g->members[(size_t)i], &e, prm, weights ? weights + lo[(size_t)i] : nullptr,
+                                                            part[(size_t)i].data(), marg, sw, cv, lev);
+        else
+            rcs[(size_t)i] = out_logev ? bnbp_run_batch_log_evidence(g->members[(size_t)i], &e, prm, marg, sw, cv, lev)
+                                       : bnbp_run_batch(g->members[(size_t)i], &e, prm, marg, sw, cv);
         if (rcs[(size_t)i]) errs[(size_t)i] = bnbp_last_error();      // the error channel is thread-local
     };
     std::vector<std::thread> threads;
@@ -2015,6 +2052,11 @@ int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* pr
     for (std::thread& t : threads) t.join();
     for (int i = 0; i < G; ++i)
         if (rcs[(size_t)i]) return fail(rcs[(size_t)i], "device " + std::to_string(g->members[(size_t)i]->device) + ": " + errs[(size_t)i]);
+    if (counts) {
+        for (int i = 1; i < G; ++i)
+            for (size_t j = 0; j < part[0].size(); ++j) part[0][j] += part[(size_t)i][j];
+        for (size_t j = 0; j < part[0].size(); ++j) counts[j] += part[0][j];
+    }
     // summary: per-case counts are still on each device (whole-shard staging of bnbp_run_batch)
     NCCL_TRY(NCCL(GroupStart)());
     for (int i = 0; i < G; ++i) {
@@ -2155,7 +2197,7 @@ void bnbp_destroy(bnbp_handle* h)
                       &h->d_pl2, &h->d_msg2[0], &h->d_msg2[1], &h->d_evbits2, &h->d_orig[0], &h->d_orig[1], &h->d_src_pos, &h->d_tile_count,
                       &h->d_evst, &h->d_lw_order, &h->d_lw_par, &h->d_lw_cpt, &h->d_lw_out, &h->d_lw_wsum, &h->d_djobs, &h->d_dytab, &h->d_ddig, &h->d_cpt_t, &h->d_tscr,
                       &h->s_ev_off, &h->s_ev_node, &h->s_ev_state, &h->s_ev_val_off, &h->s_ev_values, &h->s_out[0], &h->s_out[1], &h->s_out_all,
-                      &h->s_out_sweeps, &h->s_out_conv, &h->s_out_logev})
+                      &h->s_out_sweeps, &h->s_out_conv, &h->s_out_logev, &h->s_counts, &h->s_weights})
         b->release();
     for (auto& kv : h->belief_plans) kv.second.groups.release();
     for (cudaEvent_t e : h->ev_chunk) cudaEventDestroy(e);
@@ -2172,6 +2214,7 @@ void bnbp_destroy(bnbp_handle* h)
     if (h->pinned_poll) cudaFreeHost(h->pinned_poll);
     if (h->pin_counts) cudaFreeHost(h->pin_counts);
     if (h->pin_logev) cudaFreeHost(h->pin_logev);
+    if (h->pin_cnt) cudaFreeHost(h->pin_cnt);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
 }
@@ -2278,13 +2321,16 @@ int bnbp_spec_source(const bnbp_flat_network* net, const bnbp_options* opt, int3
     return BNBP_OK;
 }
 
+// counts_call: bnbp_run_batch_device_expected_counts (counts / weights are device memory; counts is added into by the
+// scoring launches directly).
 static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
-                            int32_t* out_sweeps, uint8_t* out_converged, double* out_logev, void* stream)
+                            int32_t* out_sweeps, uint8_t* out_converged, double* out_logev, void* stream,
+                            bool counts_call = false, double* counts = nullptr, const double* weights = nullptr)
 {
     NvtxRange nvtx_call("bnbp_run_batch_device");
     int rc = validate_params(prm);
     if (rc) return rc;
-    if (out_logev && (rc = logev_refusal(h, ev, prm, out_logev))) return rc;
+    if ((out_logev || counts_call) && (rc = logev_refusal(h, ev, prm, out_logev, counts_call, counts))) return rc;
     if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
     if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
     CU_TRY(cudaSetDevice(h->device));
@@ -2297,7 +2343,8 @@ static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_
     if (ev->n_cases == 0) return BNBP_OK;
     if (!h->members.empty()) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device: a group handle takes host buffers (bnbp_run_batch); the device path belongs to one device");
     if ((rc = set_query(h, *prm))) return rc;
-    if ((rc = choose_kernels(h, ev->n_cases, *prm, ev->ev_values != nullptr, h->precision != BNBP_FP32, out_logev != nullptr))) return rc;
+    if ((rc = choose_kernels(h, ev->n_cases, *prm, ev->ev_values != nullptr, h->precision != BNBP_FP32,
+                             out_logev != nullptr || counts_call))) return rc;
     if (!h->run_onchip && (rc = ensure_state(h, ev->n_cases))) return rc;
     // a flag left by an earlier (unchecked, asynchronous) run must not fail this one
     CU_TRY(cudaMemsetAsync(reinterpret_cast<int32_t*>(h->d_misc.p) + 1, 0, 4, st));
@@ -2334,12 +2381,13 @@ static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_
         int64_t planned = 0;
         char* const dst = out_marginals ? mine + (size_t)c0 * row_bytes : nullptr;
         double* const lev = out_logev ? out_logev + c0 : nullptr;
+        const double* const wts = weights ? weights + c0 : nullptr;
         if (h->precision == BNBP_FP32)
             rc = run_any<float, float>(h, n, de, *prm, (float*)dst, out_sweeps ? out_sweeps + c0 : nullptr,
-                                       out_converged ? out_converged + c0 : nullptr, st, &planned, lev);
+                                       out_converged ? out_converged + c0 : nullptr, st, &planned, lev, counts, wts);
         else
             rc = run_any<double, double>(h, n, de, *prm, (double*)dst, out_sweeps ? out_sweeps + c0 : nullptr,
-                                         out_converged ? out_converged + c0 : nullptr, st, &planned, lev);
+                                         out_converged ? out_converged + c0 : nullptr, st, &planned, lev, counts, wts);
         if (rc) return rc;
         if (planned < 0) exact = false; else h->last_case_sweeps += planned;
         if (exchange) {
@@ -2393,6 +2441,15 @@ int bnbp_run_batch_device_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, 
     return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, stream);
 }
 
+int bnbp_run_batch_device_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
+                                          const double* case_weights, double* counts, void* out_marginals,
+                                          int32_t* out_sweeps, uint8_t* out_converged, double* out_log_evidence, void* stream)
+{
+    if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device_expected_counts: NULL argument");
+    return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, stream, true, counts,
+                            case_weights);
+}
+
 int bnbp_check_errors(bnbp_handle* h, void* stream)
 {
     if (!h) return fail(BNBP_ERR_INVALID, "bnbp_check_errors: NULL handle");
@@ -2401,15 +2458,23 @@ int bnbp_check_errors(bnbp_handle* h, void* stream)
     return check_error_flag(h, stream ? (cudaStream_t)stream : h->stream);
 }
 
+// counts_call: bnbp_run_batch_expected_counts.  The scoring launches add into the handle's zeroed device count arena;
+// it comes back through pinned staging and is added into counts once every chunk has run.
 static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals_v,
-                          int32_t* out_sweeps, uint8_t* out_converged, double* out_logev)
+                          int32_t* out_sweeps, uint8_t* out_converged, double* out_logev, bool counts_call = false,
+                          double* counts = nullptr, const double* weights = nullptr)
 {
     const auto t_entry = std::chrono::steady_clock::now();
     NvtxRange nvtx_call("bnbp_run_batch (host buffers: H2D evidence | kernels | D2H marginals, pipelined by chunk)");
     int rc = validate_params(prm);
     if (rc) return rc;
-    if (out_logev && (rc = logev_refusal(h, ev, prm, out_logev))) return rc;
-    if (!h->members.empty()) return run_group(h, ev, prm, out_marginals_v, out_sweeps, out_converged, out_logev);
+    if ((out_logev || counts_call) && (rc = logev_refusal(h, ev, prm, out_logev, counts_call, counts))) return rc;
+    if (counts_call && weights && ev->n_cases > 0)
+        for (int64_t c = 0; c < ev->n_cases; ++c)
+            if (!(std::isfinite(weights[c]) && weights[c] >= 0.0))
+                return fail(BNBP_ERR_INVALID, "expected counts: case_weights[" + std::to_string(c) + "] is not finite and >= 0");
+    if (!h->members.empty())
+        return run_group(h, ev, prm, out_marginals_v, out_sweeps, out_converged, out_logev, counts_call ? counts : nullptr, weights);
     const bool out_f32 = prm->out_precision == BNBP_OUT_FP32;
     if (out_f32 && h->precision != BNBP_FP32)
         return fail(BNBP_ERR_INVALID, "out_precision FP32 needs an fp32 handle (an fp64 handle returns the reference's doubles)");
@@ -2435,7 +2500,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     if (ev->n_cases == 0) return BNBP_OK;
     h->reserve_sms = 0;
     if ((rc = set_query(h, *prm))) return rc;
-    if ((rc = choose_kernels(h, ev->n_cases, *prm, soft, !out_f32, out_logev != nullptr))) return rc;
+    if ((rc = choose_kernels(h, ev->n_cases, *prm, soft, !out_f32, out_logev != nullptr || counts_call))) return rc;
     if ((rc = measure_rates(h))) return rc;
     // Chunk pipeline on three streams: evidence of chunk i+1 goes up (h2d_stream) and the marginals of
     // chunk i-1 come down (copy_stream) while init/sweeps/beliefs of chunk i run.  Marginals are 8*V
@@ -2513,6 +2578,12 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
             h->pin_logev_bytes = (size_t)ev->n_cases * 8;
         }
     }
+    const size_t count_bytes = std::max<size_t>(16, (size_t)h->cpt_values * 8);
+    if (counts_call) {
+        if ((rc = h->s_counts.ensure(count_bytes))) return rc;
+        if (!h->pin_cnt) CU_TRY(cudaMallocHost((void**)&h->pin_cnt, count_bytes));
+        if (weights && (rc = h->s_weights.ensure((size_t)ev->n_cases * 8))) return rc;
+    }
     // evidence staging for the whole batch (absolute offsets, like bnbp_run_batch_device)
     if ((rc = h->s_ev_off.ensure((size_t)(ev->n_cases + 1) * 8))) return rc;
     if ((rc = h->s_ev_node.ensure(std::max<size_t>(16, (size_t)nnz * 4)))) return rc;
@@ -2541,6 +2612,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
         fprintf(stderr, "\n");
     }
     CU_TRY(cudaMemsetAsync(reinterpret_cast<int32_t*>(h->d_misc.p) + 1, 0, 4, st));
+    if (counts_call) CU_TRY(cudaMemsetAsync(h->s_counts.p, 0, count_bytes, st));
     cudaStream_t cs = h->copy_stream, hs = h->h2d_stream;
     struct Drain {                       // no path leaves this call with copies from/to host memory in flight
         cudaStream_t a, b, c;
@@ -2548,6 +2620,8 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     } drain{hs, st, cs};
     CU_TRY(cudaEventRecord(h->ev_total[0], st));
     CU_TRY(cudaStreamWaitEvent(hs, h->ev_total[0], 0));   // uploads start with the call on the device timeline
+    if (counts_call && weights)                            // ahead of every chunk's evidence: each chunk waits for those
+        CU_TRY(cudaMemcpyAsync(h->s_weights.p, weights, (size_t)ev->n_cases * 8, cudaMemcpyHostToDevice, hs));
     std::vector<cudaEvent_t> tev;                     // BNBP_TRACE: device timeline of the pipeline
     auto mark = [&](cudaStream_t s) {
         if (!trace) return;
@@ -2602,15 +2676,17 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
         CU_TRY(cudaStreamWaitEvent(st, e_up, 0));
         char* slot = !out_marginals ? nullptr : whole ? (char*)h->s_out_all.p + (size_t)c0 * row_bytes : (char*)h->s_out[idx & 1].p;
         double* const lev = out_logev ? (double*)h->s_out_logev.p + c0 : nullptr;
+        double* const cnt = counts_call ? (double*)h->s_counts.p : nullptr;
+        const double* const wts = counts_call && weights ? (const double*)h->s_weights.p + c0 : nullptr;
         if (!whole && idx >= 2) CU_TRY(cudaStreamWaitEvent(st, h->ev_chunk[3 * (idx - 2) + 2], 0));   // ring slot is free again
         stamp("enqueue chunk", idx);
         mark(st);
         if (h->precision == BNBP_FP32 && out_f32)
-            rc = run_any<float, float>(h, n, de, *prm, (float*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev);
+            rc = run_any<float, float>(h, n, de, *prm, (float*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev, cnt, wts);
         else if (h->precision == BNBP_FP32)
-            rc = run_any<float, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev);
+            rc = run_any<float, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev, cnt, wts);
         else
-            rc = run_any<double, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev);
+            rc = run_any<double, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev, cnt, wts);
         if (rc) return rc;
         mark(st);
         CU_TRY(cudaEventRecord(e_done, st));
@@ -2634,6 +2710,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     // copy_stream is in order: everything before e_last has left when it fires
     stamp("all enqueued", idx);
     // the call returns with every result on the host
+    if (counts_call) CU_TRY(cudaMemcpyAsync(h->pin_cnt, h->s_counts.p, count_bytes, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamWaitEvent(st, e_last, 0));
     CU_TRY(cudaEventRecord(h->ev_total[1], st));
     h->total_recorded = true;
@@ -2641,6 +2718,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     NvtxRange nvtx_wait("bnbp: wait for the streams");
     if ((rc = check_error_flag(h, st))) return rc;
     CU_TRY(wait_stream(cs));
+    if (counts_call) CU_TRY(wait_stream(st));
     h->last_host_wait_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_wait).count();
     stamp("done", idx);
     for (size_t i = 0; i + 3 < tev.size(); i += 4) {
@@ -2655,6 +2733,8 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     if (out_sweeps) memcpy(out_sweeps, pin_sweeps, (size_t)ev->n_cases * 4);
     if (out_converged) memcpy(out_converged, pin_conv, (size_t)ev->n_cases);
     if (out_logev) memcpy(out_logev, h->pin_logev, (size_t)ev->n_cases * 8);
+    if (counts_call)
+        for (int64_t j = 0; j < h->cpt_values; ++j) counts[j] += h->pin_cnt[j];
     if (!(prm->epsilon > 0.0)) {
         h->last_case_sweeps = ev->n_cases * (int64_t)prm->max_sweeps;     // fixed count: every case ran them all
     } else if (out_sweeps) {
@@ -2680,6 +2760,14 @@ int bnbp_run_batch_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const b
 {
     if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_log_evidence: NULL argument");
     return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence);
+}
+
+int bnbp_run_batch_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
+                                   const double* case_weights, double* counts, void* out_marginals, int32_t* out_sweeps,
+                                   uint8_t* out_converged, double* out_log_evidence)
+{
+    if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_expected_counts: NULL argument");
+    return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, true, counts, case_weights);
 }
 
 int bnbp_lw_run_batch(bnbp_handle* h, const bnbp_evidence* ev, int64_t n_samples, uint64_t seed, double* out_marginals,

@@ -68,6 +68,7 @@ class BPResult:
     sweeps: np.ndarray         # [n_cases] int32
     converged: np.ndarray      # [n_cases] uint8
     log_evidence: Optional[np.ndarray] = None   # [n_cases] float64, Bethe estimate of ln P(e) (log_evidence=True)
+    expected_counts: Optional[np.ndarray] = None   # [cpt_values] float64, expected family counts (expected_counts=True)
 
     def node(self, net: FlatNetwork, x: int) -> np.ndarray:
         off = net.belief_off
@@ -76,6 +77,35 @@ class BPResult:
 
 def _vp(a) -> Optional[int]:
     return None if a is None else a.ctypes.data
+
+
+def m_step(net: FlatNetwork, counts: np.ndarray, pseudo_count: float = 0.0) -> np.ndarray:
+    """The M-step of EM: ``sampler::make_cpt``'s normalisation (sampler.hpp:147-163) of expected family counts in the
+    CPT-arena layout of ``net`` (``BPResult.expected_counts``).  ``pseudo_count`` is added to every entry first; a row
+    whose total is 0 becomes uniform 1/r, as make_cpt does for a parent configuration never seen."""
+    counts = np.asarray(counts, dtype=np.float64)
+    if counts.shape != (int(net.cpt_off[-1]),):
+        raise ValueError("counts must have cpt_off[-1] entries")
+    if not (np.isfinite(pseudo_count) and pseudo_count >= 0.0):
+        raise ValueError("pseudo_count must be finite and >= 0")
+    out = np.empty_like(counts)
+    for x in range(net.n_nodes):
+        a, b, r = int(net.cpt_off[x]), int(net.cpt_off[x + 1]), int(net.card[x])
+        rows = counts[a:b].reshape(-1, r) + pseudo_count
+        tot = rows.sum(axis=1, keepdims=True)
+        zero = tot[:, 0] == 0.0
+        dst = out[a:b].reshape(-1, r)
+        dst[~zero] = rows[~zero] / tot[~zero]
+        dst[zero] = 1.0 / r
+    return out
+
+
+@dataclass
+class EMResult:
+    cpt: np.ndarray                # [cpt_values] the CPT after the last M-step (the handle holds it)
+    log_likelihood: np.ndarray     # [iterations] sum_c w_c ln Z_B(e_c) over the counted cases, under the CPT going in
+    skipped: np.ndarray            # [iterations] cases whose evidence was impossible under that CPT (counted nowhere)
+    iterations: int
 
 
 class BeliefPropagation:
@@ -126,16 +156,22 @@ class BeliefPropagation:
                  out: Optional[np.ndarray] = None, out_sweeps: Optional[np.ndarray] = None,
                  out_converged: Optional[np.ndarray] = None, query_nodes: Optional[Sequence[int]] = None,
                  out_dtype=np.float64, semiring: str = "sum", log_evidence: bool = False,
-                 marginals: bool = True) -> BPResult:
+                 marginals: bool = True, expected_counts: bool = False, weights: Optional[np.ndarray] = None,
+                 counts_out: Optional[np.ndarray] = None) -> BPResult:
         """``query_nodes``: only these nodes' marginals are returned (columns in the given order);
         ``out_dtype=np.float32`` (fp32 handles): float marginals, half the device-to-host copy;
         ``semiring="max"``: max-product (max-marginals) instead of the reference's sum-product;
         ``log_evidence=True``: also each case's Bethe estimate of ln P(e) (``bnbp_run_batch_log_evidence``; exact on
         polytrees run to convergence; hard evidence only) in ``BPResult.log_evidence``;
-        ``marginals=False`` (with ``log_evidence``): no marginals are computed into or copied to the host, the result's
-        marginals are an (n, 0) array."""
-        if not marginals and not log_evidence:
-            raise ValueError("marginals=False needs log_evidence=True (the call would return nothing)")
+        ``marginals=False`` (with ``log_evidence`` or ``expected_counts``): no marginals are computed into or copied to
+        the host, the result's marginals are an (n, 0) array;
+        ``expected_counts=True``: also the E-step of EM (``bnbp_run_batch_expected_counts``): sum_c w_c P(x, u | e_c)
+        per CPT entry from the family beliefs of the final state, in ``BPResult.expected_counts`` (CPT-arena layout;
+        ``weights`` [n_cases], default 1; added into ``counts_out`` when given, else into zeros)."""
+        if not marginals and not log_evidence and not expected_counts:
+            raise ValueError("marginals=False needs log_evidence=True or expected_counts=True (the call would return nothing)")
+        if not expected_counts and (weights is not None or counts_out is not None):
+            raise ValueError("weights / counts_out belong to expected_counts=True")
         if evidence is None:
             evidence = EvidenceBatch.empty(1)   # operator()(epsilon) by-pass (:24-28)
         ev = evidence
@@ -164,6 +200,18 @@ class BeliefPropagation:
         prm = _capi.RunParamsC(float(epsilon), int(max_sweeps), float(damping), int(check_interval),
                                2 if out_dtype == np.float32 else 0, 0, 0 if q is None else int(q.size), _vp(q),
                                {"sum": 0, "max": 1}[semiring])
+        if expected_counts:
+            nv = int(self.net.cpt_off[-1])
+            counts = np.zeros(nv, dtype=np.float64) if counts_out is None else counts_out
+            assert counts.dtype == np.float64 and counts.size == nv and counts.flags.c_contiguous
+            w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
+            if w is not None and w.shape != (n,):
+                raise ValueError("weights must be [n_cases]")
+            logev = np.empty(n, dtype=np.float64) if log_evidence else None
+            _capi.check(self._lib.bnbp_run_batch_expected_counts(self._h, C.byref(evc), C.byref(prm), _vp(w), _vp(counts),
+                                                                 _vp(out) if marginals else None, _vp(sweeps), _vp(conv),
+                                                                 _vp(logev)))
+            return BPResult(out.reshape(n, V if marginals else 0), sweeps, conv, logev, counts)
         if log_evidence:
             logev = np.empty(n, dtype=np.float64)
             _capi.check(self._lib.bnbp_run_batch_log_evidence(self._h, C.byref(evc), C.byref(prm),
@@ -177,12 +225,16 @@ class BeliefPropagation:
     def run_device(self, n_cases: int, ev_off, ev_node, ev_state, out, *, ev_val_off=None, ev_values=None,
                    epsilon: float = 0.0, max_sweeps: int = 20, damping: float = 0.0, check_interval: int = 1,
                    out_sweeps=None, out_converged=None, stream: int = 0, gather: bool = False,
-                   query_nodes: Optional[Sequence[int]] = None, out_log_evidence=None) -> None:
+                   query_nodes: Optional[Sequence[int]] = None, out_log_evidence=None, out_counts=None,
+                   case_weights=None) -> None:
         """All tensor arguments are CUDA tensors (int64 / int32 / float64 offsets and values as in
         ``bnbp_evidence``); ``out`` has the handle's precision, shape [n_cases, sum r_X].
         Work is enqueued on ``stream`` (a raw cudaStream_t, e.g. torch.cuda.current_stream().cuda_stream).
         ``out_log_evidence``: a float64 CUDA tensor [n_cases] that receives each case's Bethe log-evidence
-        (``bnbp_run_batch_device_log_evidence``); ``out`` may then be None (no marginals)."""
+        (``bnbp_run_batch_device_log_evidence``); ``out`` may then be None (no marginals).
+        ``out_counts``: a float64 CUDA tensor [cpt_values] that the expected family counts are ADDED into, in stream
+        order (``bnbp_run_batch_device_expected_counts``), with ``case_weights`` a float64 CUDA tensor [n_cases] (finite
+        and >= 0, not checked) or None; ``out`` and ``out_log_evidence`` may then be None."""
         def dp(t):
             return None if t is None else int(t.data_ptr())
         evc = _capi.EvidenceC(int(n_cases), dp(ev_off), dp(ev_node), dp(ev_state), dp(ev_val_off), dp(ev_values))
@@ -192,6 +244,17 @@ class BeliefPropagation:
         prm = _capi.RunParamsC(float(epsilon), int(max_sweeps), float(damping), int(check_interval), 0,
                                1 if gather else 0, 0 if q is None else int(q.size), _vp(q))
         st = C.c_void_p(stream) if stream else None
+        if out_counts is not None or case_weights is not None:
+            if out_counts is None:
+                raise ValueError("case_weights belong to out_counts")
+            for t, m in ((out_counts, int(self.net.cpt_off[-1])), (case_weights, int(n_cases)),
+                         (out_log_evidence, int(n_cases))):
+                if t is not None:
+                    assert t.dtype.itemsize == 8 and t.is_floating_point() and t.is_cuda and t.numel() == m and t.is_contiguous()
+            _capi.check(self._lib.bnbp_run_batch_device_expected_counts(self._h, C.byref(evc), C.byref(prm), dp(case_weights),
+                                                                        dp(out_counts), dp(out), dp(out_sweeps),
+                                                                        dp(out_converged), dp(out_log_evidence), st))
+            return
         if out_log_evidence is not None:
             assert out_log_evidence.dtype.itemsize == 8 and out_log_evidence.is_floating_point() and out_log_evidence.is_cuda
             assert out_log_evidence.numel() == int(n_cases) and out_log_evidence.is_contiguous()
@@ -259,6 +322,41 @@ class BeliefPropagation:
     def refresh_cpt(self, cpt: np.ndarray) -> None:
         cpt = np.ascontiguousarray(cpt, dtype=np.float64)
         _capi.check(self._lib.bnbp_refresh_cpt(self._h, _vp(cpt), cpt.size))
+
+    # ---- EM parameter learning from incomplete evidence -----------------------------------------------
+    def em(self, evidence: EvidenceBatch, *, iterations: int = 50, tol: float = 1e-6, pseudo_count: float = 0.0,
+           epsilon: float = 1e-6, max_sweeps: int = 200, damping: float = 0.0,
+           weights: Optional[np.ndarray] = None, cpt: Optional[np.ndarray] = None) -> EMResult:
+        """Expectation-maximisation of the CPTs from the hard-evidence cases ``evidence`` (``weights`` [n_cases]: each
+        case's multiplicity, default 1).  Each iteration: the E-step on the GPU (expected family counts and the Bethe
+        log-evidence of every case, one ``expected_counts`` call), ``m_step`` on the host and ``refresh_cpt``.  Starts
+        from ``cpt`` (default ``self.net.cpt``; ``self.net`` is never modified) and stops after ``iterations`` or once
+        the log-likelihood gains no more than ``tol * |L|``.  ``log_likelihood[i]`` is sum_c w_c ln Z_B(e_c) over the
+        cases counted in iteration i, under the CPT going into it (exact on polytrees run to convergence, the Bethe
+        approximation on loopy networks).  The handle is left holding the returned CPT."""
+        if iterations < 1:
+            raise ValueError("iterations must be >= 1")
+        n = evidence.n_cases
+        w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
+        if w is not None and (w.shape != (n,) or not np.isfinite(w).all() or (w < 0).any()):
+            raise ValueError("weights must be [n_cases], finite and >= 0")
+        cur = np.array(self.net.cpt if cpt is None else cpt, dtype=np.float64)
+        self.refresh_cpt(cur)            # the handle may hold another CPT from an earlier refresh_cpt
+        counts = np.zeros(int(self.net.cpt_off[-1]), dtype=np.float64)
+        lls, skipped = [], []
+        for it in range(iterations):
+            counts[:] = 0.0
+            res = self(evidence, epsilon, max_sweeps=max_sweeps, damping=damping, marginals=False, log_evidence=True,
+                       expected_counts=True, weights=w, counts_out=counts)
+            ok = np.isfinite(res.log_evidence)
+            le = res.log_evidence[ok]
+            lls.append(float(le.sum() if w is None else (w[ok] * le).sum()))
+            skipped.append(int((~ok).sum()))
+            cur = m_step(self.net, counts, pseudo_count)
+            self.refresh_cpt(cur)
+            if it > 0 and lls[-1] - lls[-2] <= tol * abs(lls[-1]):
+                break
+        return EMResult(cur, np.array(lls), np.array(skipped, dtype=np.int64), len(lls))
 
 
 # the name the north star uses (SURVEY.md section 0.1: the reference class is belief_propagation)

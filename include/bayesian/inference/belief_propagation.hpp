@@ -116,6 +116,7 @@ public:
         std::vector<vertex_type> query;   // non-empty: only these vertices' marginals, in this order
         bool float_marginals = false;     // fp32 handles: marginals_f32 is filled instead of marginals (half the copy)
         bool log_evidence = false;        // flat_result::log_evidence: each case's Bethe estimate of ln P(e) (hard evidence)
+        bool expected_counts = false;     // flat_result::expected_counts: the E-step of EM (bnbp_run_batch_expected_counts)
     };
 
     struct flat_result {
@@ -128,6 +129,10 @@ public:
         pinned_buffer<std::int32_t> sweeps;        // sweeps executed per case
         pinned_buffer<std::uint8_t> converged;     // 1 if the case met delta < epsilon
         std::vector<double> log_evidence;          // options::log_evidence: per case (bnbp_run_batch_log_evidence), else empty
+        // options::expected_counts: sum over the cases of P(x, u | e) per CPT entry, in the flat CPT arena of the graph
+        // (vertex_list() order, rows by parent configuration, last parent fastest; each row normalised is the M-step,
+        // written back through the vertices' cpt_t and picked up by the next call), else empty
+        std::vector<double> expected_counts;
         bnbp_summary summary = bnbp_summary();     // totals over all devices (devices.size() > 1: all-reduced over NCCL)
     };
 
@@ -335,13 +340,20 @@ private:
         prm.semiring = opt.semiring;
         prm.n_query = static_cast<std::int32_t>(query.size());
         prm.query_nodes = query.empty() ? nullptr : query.data();
-        if (opt.log_evidence) {
-            out.log_evidence.resize(out.n_cases);
+        if (opt.log_evidence) out.log_evidence.resize(out.n_cases);
+        else out.log_evidence.clear();
+        if (opt.expected_counts) {
+            out.expected_counts.assign(flat_.cpt.size(), 0.0);
+            if (bnbp_run_batch_expected_counts(handle_, &ev, &prm, nullptr, out.expected_counts.data(), dst, out.sweeps.data(),
+                                               out.converged.data(), opt.log_evidence ? out.log_evidence.data() : nullptr) != BNBP_OK)
+                throw std::runtime_error(last_error("bnbp_run_batch_expected_counts"));
+        } else if (opt.log_evidence) {
+            out.expected_counts.clear();
             if (bnbp_run_batch_log_evidence(handle_, &ev, &prm, dst, out.sweeps.data(), out.converged.data(),
                                             out.log_evidence.data()) != BNBP_OK)
                 throw std::runtime_error(last_error("bnbp_run_batch_log_evidence"));
         } else {
-            out.log_evidence.clear();
+            out.expected_counts.clear();
             if (bnbp_run_batch(handle_, &ev, &prm, dst, out.sweeps.data(), out.converged.data()) != BNBP_OK)
                 throw std::runtime_error(last_error("bnbp_run_batch"));
         }
@@ -354,6 +366,7 @@ private:
         opt.query.clear();
         opt.float_marginals = false;
         opt.log_evidence = false;
+        opt.expected_counts = false;
         return opt;
     }
 

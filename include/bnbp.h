@@ -19,6 +19,7 @@
  *   bnbp_host_alloc/free  (new: page-locked result buffers for bnbp_run_batch)
  *   bnbp_check_errors  (evidence validation of the asynchronous device-path call; no reference counterpart)
  *   bnbp_run_batch_log_evidence / bnbp_run_batch_device_log_evidence  (new: per-case Bethe log-evidence)
+ *   bnbp_run_batch_expected_counts / bnbp_run_batch_device_expected_counts  (new: the E-step of EM)
  *   bnbp_destroy       <- belief_propagation::~belief_propagation()   :21
  *   bnbp_last_error    <- (the reference has no error channel; UB / NaN / endless loop)
  *   bnbp_refresh_cpt   <- the reference reads vertex_t::cpt at call time (graph.hpp:157-161), so
@@ -293,6 +294,32 @@ int  bnbp_run_batch_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const 
 int  bnbp_run_batch_device_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
                                         void* out_marginals, int32_t* out_sweeps, uint8_t* out_converged,
                                         double* out_log_evidence, void* stream);
+
+/* Expected family counts (no reference counterpart): the E-step of EM parameter learning from incomplete evidence.
+ * The run of bnbp_run_batch_log_evidence, whose scoring launches also add, for every case c of weight w_c (1 when
+ * case_weights is NULL) with a finite log-evidence, the family posterior b_X of the log-evidence above into counts:
+ *   counts[cpt_off[X] + q r_X + x] += w_c P(x|u_q) lambda_X(x) prod_j pm_j(u_qj) / Z_X      for every X, q, x
+ * with lambda_X and pm_j of the case's last executed sweep as above.  counts has the layout of the CPT arena
+ * (cpt_off[n_nodes] doubles), so sampler::make_cpt's normalisation of each row is the M-step.  A case whose
+ * log-evidence is NaN or -inf (some Z_X is NaN or 0: the evidence is impossible under the CPT) adds nothing; it still
+ * gets its log-evidence, sweeps and flag.  Summed over x and u the counts of a node are sum_c w_c b_X(x), the node
+ * marginal, at any sweep count; on a polytree run to its fixed point they are sum_c w_c P(x, u | e_c).
+ * The call ADDS INTO counts: zero it once and stream a data set larger than one call through several calls before
+ * an M-step.  Sums are fp64 in both precisions, but atomics leave their order open: counts agree between runs to
+ * rounding, not bit for bit.  case_weights [n_cases] must be finite and >= 0 (the host call checks this and refuses
+ * otherwise; the device call reads them as given).  case_weights, out_marginals and out_log_evidence may be NULL.
+ * Host call: host buffers, the handle's own zeroed device count arena is added into counts when the call returns;
+ * group handles add the members' counts in member order.  Device call: device pointers, counts is added into on
+ * the device, in stream order.  Kernels and refusals are log-evidence's, plus BNBP_ERR_INVALID for a NULL counts;
+ * the handle stays usable after a refusal. */
+int  bnbp_run_batch_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
+                                    const double* case_weights, double* counts,
+                                    void* out_marginals, int32_t* out_sweeps, uint8_t* out_converged,
+                                    double* out_log_evidence);
+int  bnbp_run_batch_device_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
+                                           const double* case_weights, double* counts,
+                                           void* out_marginals, int32_t* out_sweeps, uint8_t* out_converged,
+                                           double* out_log_evidence, void* stream);
 
 /* Likelihood weighting for a batch of HARD-evidence cases (SURVEY 8 f2): the independent statistical
  * check of BP marginals on loopy networks.  Replaces likelihood_weighting::operator()(evidence_list,

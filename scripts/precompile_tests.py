@@ -64,6 +64,10 @@ def jobs():
         out.append((net, "fp64", (1 << 8) | (1 << 10), unrolled))
         out.append((net, "fp32", 1 << 9, unrolled))
     out.append((en.catalogue()["hub65"], "fp64", 0b01111111))
+    # expected counts (tests/test_gpu_em.py): the polytree checked against enumeration, and the 20 x 20 grid class-looped
+    for prec in ("fp64", "fp32"):
+        out.append((synth.random_polytree(8, card_hi=4, max_parents=3, seed=9), prec, 0b11111))
+        out.append((synth.grid(20), prec, 0b11001, force))
     return out
 
 
