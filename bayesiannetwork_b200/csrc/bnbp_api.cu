@@ -138,9 +138,15 @@ struct NvtxRange {
 
 constexpr int BLOCK_THREADS = 128;   // sweep-kernel block; a tile holds BLOCK_THREADS * vec cases
 
+// Device memory that grows on demand and is freed by its destructor (a handle's buffers: by `delete h` in
+// bnbp_destroy, while the handle's device is current).
 struct DevBuf {
     void* p = nullptr;
     size_t bytes = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { release(); }
     int ensure(size_t need)
     {
         if (need <= bytes) return BNBP_OK;
@@ -156,6 +162,26 @@ struct DevBuf {
         if (p) cudaFree(p);
         p = nullptr;
         bytes = 0;
+    }
+};
+
+// The same for pinned host memory (staging of device-to-host copies)
+struct PinnedBuf {
+    void* p = nullptr;
+    size_t bytes = 0;
+    PinnedBuf() = default;
+    PinnedBuf(const PinnedBuf&) = delete;
+    PinnedBuf& operator=(const PinnedBuf&) = delete;
+    ~PinnedBuf() { if (p) cudaFreeHost(p); }
+    int ensure(size_t need)
+    {
+        if (need <= bytes) return BNBP_OK;
+        if (p) cudaFreeHost(p);
+        p = nullptr;
+        bytes = 0;
+        CU_TRY(cudaMallocHost(&p, need));
+        bytes = need;
+        return BNBP_OK;
     }
 };
 
@@ -258,18 +284,16 @@ struct bnbp_handle {
     std::vector<int32_t> par_host;
     DevBuf d_lw_order, d_lw_par, d_lw_cpt, d_lw_out, d_lw_wsum;
     bool lw_ready = false;
-    void* pin_counts = nullptr;         // pinned host staging of the per-case sweep counts / converged flags
-    size_t pin_counts_bytes = 0;
+    PinnedBuf pin_counts;               // pinned host staging of the per-case sweep counts / converged flags
     DevBuf s_out_logev;                 // log-evidence of the whole batch (host-buffer call), and its pinned staging
-    double* pin_logev = nullptr;
-    size_t pin_logev_bytes = 0;
+    PinnedBuf pin_logev;
     DevBuf s_counts, s_weights;         // expected-counts call (host buffers): the call's zeroed count arena, the weights
-    double* pin_cnt = nullptr;          // pinned staging of the count arena (cpt_values doubles)
+    PinnedBuf pin_cnt;                  // pinned staging of the count arena (cpt_values doubles)
     DevBuf s_out_all;                   // whole-batch output staging (used when HBM has the room)
     cudaStream_t copy_stream = nullptr, h2d_stream = nullptr;
     std::vector<cudaEvent_t> ev_chunk;  // per chunk of the host-buffer call: uploaded, computed, copied
     // column groups of the tiled belief kernel, per (tile width, output element size)
-    struct BeliefPlan { DevBuf groups; int n_groups = 0; int stride = 0; size_t smem = 0; bool ok = false; };
+    struct BeliefPlan { DevBuf groups; int n_groups = 0; int stride = 0; size_t smem = 0; };
     std::map<int, BeliefPlan> belief_plans;
     int32_t* pinned_poll = nullptr;    // [4]
     cudaStream_t stream = nullptr;
@@ -295,7 +319,7 @@ struct bnbp_handle {
     cudaStream_t comm_stream = nullptr;
     std::vector<cudaEvent_t> ev_comm;  // per gather chunk: computed, gathered
     DevBuf d_summary;                  // 4 x int64: case sweeps, not converged, max sweeps, cases
-    int64_t* pin_summary = nullptr;    // pinned [4]
+    PinnedBuf pin_summary;             // 8 x int64 (the totals of d_summary)
     std::vector<bnbp_handle*> members; // group handle: one member per device (the group itself holds no device state)
     bnbp_summary last_summary = {0, 0, 0, 0};
 };
@@ -617,13 +641,12 @@ int belief_plan(bnbp_handle* h, int tb, int out_size, bnbp_handle::BeliefPlan** 
         g.n1 = x; g.j1 = g.j0 + w;
         groups.push_back(g);
     }
-    p.ok = true;
-    p.n_groups = (int)groups.size();
-    p.stride = width | 1;                                // odd row stride: conflict-free phase 1
-    p.smem = (size_t)tb * p.stride * out_size;           // tb/32 warps x [32][stride]
     int rc = p.groups.ensure(groups.size() * sizeof(BeliefGroup));
     if (rc) return rc;
     CU_TRY(cudaMemcpy(p.groups.p, groups.data(), groups.size() * sizeof(BeliefGroup), cudaMemcpyHostToDevice));
+    p.stride = width | 1;                                // odd row stride: conflict-free phase 1
+    p.smem = (size_t)tb * p.stride * out_size;           // tb/32 warps x [32][stride]
+    p.n_groups = (int)groups.size();                     // the plan is complete: later calls take it as it is
     return BNBP_OK;
 }
 
@@ -633,14 +656,39 @@ struct DevEvidence {       // device pointers, offsets absolute with the given b
     const int64_t* ev_val_off; const double* ev_values; int64_t ev_val_base;
 };
 
+// What a batch call writes (NULL: not asked for) and which entry point made the call.  The per-case arrays start at
+// the first case of the call; counts is one array (layout of the CPT arena) that the call adds into.
+struct RunOutputs {
+    enum Entry { PLAIN, LOG_EVIDENCE, EXPECTED_COUNTS };
+    Entry entry = PLAIN;
+    void* marginals = nullptr;
+    int32_t* sweeps = nullptr;
+    uint8_t* converged = nullptr;
+    double* logev = nullptr;
+    double* counts = nullptr;
+    const double* weights = nullptr;        // per case, NULL = 1 (expected counts)
+    // the run also scores each case (log_evidence_kernel), so choose_kernels leaves out what cannot score
+    bool scored() const { return logev || entry == EXPECTED_COUNTS; }
+    // the outputs of the cases from c0 on (marginal rows of row_bytes)
+    RunOutputs at(int64_t c0, size_t row_bytes) const
+    {
+        RunOutputs o = *this;
+        if (marginals) o.marginals = (char*)marginals + (size_t)c0 * row_bytes;
+        if (sweeps) o.sweeps += c0;
+        if (converged) o.converged += c0;
+        if (logev) o.logev += c0;
+        if (weights) o.weights += c0;
+        return o;
+    }
+};
+
 // log_evidence_kernel over the positions [0, n_pos) of an arena (arguments as belief_tiled_kernel's).  Blocks are as
 // wide as the per-thread accumulator columns allow in 96 KB of shared memory (at least one warp: r <= 128).
-// d_counts: the kernel's count pass also adds each scored case's family posteriors (weights d_weights, NULL = 1) into
-// it; d_out_logev may then be NULL.
+// out.counts: the kernel's count pass also adds each scored case's family posteriors (weights out.weights) into it;
+// out.logev may then be NULL.  The kernel writes the sweep counts and flags when no marginals are written.
 template <typename T>
 int launch_logev(bnbp_handle* h, const T* pl, T* const (&msg)[2], int64_t n_pos, const int32_t* orig, int only_frozen,
-                 double* d_out_logev, int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st,
-                 double* d_counts = nullptr, const double* d_weights = nullptr)
+                 const RunOutputs& out, cudaStream_t st)
 {
     int vals = 1;
     for (int x = 0; x < h->N; ++x) {
@@ -648,40 +696,50 @@ int launch_logev(bnbp_handle* h, const T* pl, T* const (&msg)[2], int64_t n_pos,
         for (int j = 0; j < h->nodes[x].k; ++j) rj = std::max(rj, (int)h->e_card[(size_t)h->nodes[x].e0 + j]);
         vals = std::max(vals, h->nodes[x].card + rj);
     }
-    if (d_counts) vals += 1;                                // + one reduction slot per thread (32 entries per warp)
+    if (out.counts) vals += 1;                              // + one reduction slot per thread (32 entries per warp)
     const int threads = std::max(32, std::min(256, (int)(96 * 1024 / (vals * 8)) / 32 * 32));
     const size_t smem = (size_t)threads * vals * 8;
     const unsigned blocks = (unsigned)((n_pos + threads - 1) / threads);
-    if (d_counts) {
-        if (smem > 48 * 1024)
-            CU_TRY(cudaFuncSetAttribute(log_evidence_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        log_evidence_kernel<T, true><<<blocks, threads, smem, st>>>(
-            (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
-            h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
-            d_out_logev, d_out_sweeps, d_out_conv, d_weights, d_counts);
-    } else {
-        if (smem > 48 * 1024)
-            CU_TRY(cudaFuncSetAttribute(log_evidence_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        log_evidence_kernel<T, false><<<blocks, threads, smem, st>>>(
-            (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
-            h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
-            d_out_logev, d_out_sweeps, d_out_conv, nullptr, nullptr);
-    }
+    const auto kernel = out.counts ? log_evidence_kernel<T, true> : log_evidence_kernel<T, false>;
+    if (smem > 48 * 1024)
+        CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<blocks, threads, smem, st>>>(
+        (const NodeMeta*)h->d_nodes.p, h->N, (const int32_t*)h->d_e_card.p, (const T*)h->d_cpt.p, pl, msg[0], msg[1],
+        h->PL, h->M, h->tb, n_pos, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, orig, only_frozen,
+        out.logev, out.marginals ? nullptr : out.sweeps, out.marginals ? nullptr : out.converged,
+        out.counts ? out.weights : nullptr, out.counts);
     CU_TRY(cudaGetLastError());
     h->last_kernel_launches++;
     return BNBP_OK;
 }
 
-// Runs init -> sweeps -> beliefs for n (<= cap) cases whose evidence is on the device.  d_out_logev: also the
-// log-evidence of each case (choose_kernels was told); d_out may then be NULL (no marginals).  d_counts: the same
-// scoring launches also add the expected family counts into it (weights d_weights of this chunk's cases, NULL = 1);
-// d_out_logev may then be NULL.
+// belief_tiled_kernel over the positions [0, n_pos) of an arena, into out.marginals (orig, only_frozen: as the kernel's)
 template <typename T, typename OUT>
-int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out,
-              int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps,
-              double* d_out_logev = nullptr, double* d_counts = nullptr, const double* d_weights = nullptr)
+int launch_beliefs(bnbp_handle* h, const T* pl, int64_t n_pos, const int32_t* orig, int only_frozen, const RunOutputs& out,
+                   cudaStream_t st)
 {
-    const bool scored = d_out_logev || d_counts;
+    bnbp_handle::BeliefPlan* plan = nullptr;
+    const int rc = belief_plan(h, h->tb, (int)sizeof(OUT), &plan);
+    if (rc) return rc;
+    if (plan->smem > 48 * 1024)
+        CU_TRY(cudaFuncSetAttribute(belief_tiled_kernel<T, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan->smem));
+    belief_tiled_kernel<T, OUT><<<(unsigned)((n_pos + h->tb - 1) / h->tb), h->tb, plan->smem, st>>>(
+        (const NodeMeta*)h->d_nodes.p, (const BeliefGroup*)plan->groups.p, plan->n_groups, pl, h->PL, h->tb, h->V,
+        plan->stride, n_pos, (OUT*)out.marginals, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p, out.sweeps,
+        out.converged, orig, only_frozen);
+    CU_TRY(cudaGetLastError());
+    h->last_kernel_launches++;
+    return BNBP_OK;
+}
+
+// Runs init -> sweeps -> beliefs for n (<= cap) cases whose evidence is on the device, into the device arrays of out.
+// out.scored(): also the log-evidence of each case and / or the expected family counts (choose_kernels was told);
+// out.marginals may then be NULL.
+template <typename T, typename OUT>
+int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, const RunOutputs& out,
+              cudaStream_t st, int64_t* planned_sweeps)
+{
+    OUT* const d_out = (OUT*)out.marginals;
     NvtxRange nvtx_chunk("bnbp: chunk (init, sweeps, beliefs) streaming kernels");
     const int tiles = (int)((n + h->tb - 1) / h->tb);
     int32_t* d_last_active = reinterpret_cast<int32_t*>(h->d_misc.p);
@@ -928,7 +986,7 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
                 CU_TRY(cudaMemsetAsync(d_total, 0, 4, st));
                 delta_retire_kernel<T, OUT><<<tiles_cur, h->tb, 0, st>>>(
                     (const NodeMeta*)h->d_nodes.p, h->N, h->PL, h->M, h->V, pl_p, sa.msg_cur, sa.msg_nxt, (uint8_t*)h->d_status.p,
-                    (T)prm.epsilon, t + 1, n_cur, orig, d_out, d_out_sweeps, d_out_conv, (int32_t*)h->d_tile_count.p, d_total);
+                    (T)prm.epsilon, t + 1, n_cur, orig, d_out, out.sweeps, out.converged, (int32_t*)h->d_tile_count.p, d_total);
                 CU_TRY(cudaGetLastError());
                 h->last_kernel_launches++;
                 have_total = true;
@@ -989,23 +1047,9 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
                              h->d_src_pos.ensure((size_t)h->cap * 4)))
                     fits = false;
                 if (fits && split) have_total = false;           // the counts describe the old arena
-                if (fits && !split && d_out) {
-                    // 1. retire the converged cases: their state is final (:135-147), write their beliefs now
-                    bnbp_handle::BeliefPlan* plan = nullptr;
-                    if ((rc = belief_plan(h, h->tb, (int)sizeof(OUT), &plan))) return rc;
-                    if (plan->smem > 48 * 1024)
-                        CU_TRY(cudaFuncSetAttribute(belief_tiled_kernel<T, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan->smem));
-                    belief_tiled_kernel<T, OUT><<<tiles_cur, h->tb, plan->smem, st>>>(
-                        (const NodeMeta*)h->d_nodes.p, (const BeliefGroup*)plan->groups.p, plan->n_groups, pl_p, h->PL,
-                        h->tb, h->V, plan->stride, n_cur, d_out, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p,
-                        d_out_sweeps, d_out_conv, orig, 1);
-                    CU_TRY(cudaGetLastError());
-                    h->last_kernel_launches++;
-                }
-                if (fits && !split && scored &&
-                    (rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 1, d_out_logev, d_out ? nullptr : d_out_sweeps,
-                                          d_out ? nullptr : d_out_conv, st, d_counts, d_weights)))
-                    return rc;
+                // 1. retire the converged cases: their state is final (:135-147), write their beliefs now
+                if (fits && !split && d_out && (rc = launch_beliefs<T, OUT>(h, pl_p, n_cur, orig, 1, out, st))) return rc;
+                if (fits && !split && out.scored() && (rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 1, out, st))) return rc;
                 if (fits) {
                     // 2. new position -> old position (stable), 3. gather into the other arena
                     compact_scan_kernel<<<1, 1024, 0, st>>>(d_tile_cnt, d_tile_off, tiles_cur);
@@ -1069,34 +1113,18 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
 
     if (fuse) {
         // K4 ran inside the last sweep (variants 6/7); only the per-case counts are left
-        if (d_out_sweeps || d_out_conv) {
+        if (out.sweeps || out.converged) {
             counts_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p,
-                                                                        d_out_sweeps, d_out_conv, n);
+                                                                        out.sweeps, out.converged, n);
             CU_TRY(cudaGetLastError());
             h->last_kernel_launches++;
         }
     } else if (d_out) {
-        bnbp_handle::BeliefPlan* plan = nullptr;
-        int rc = belief_plan(h, h->tb, (int)sizeof(OUT), &plan);
+        const int rc = launch_beliefs<T, OUT>(h, pl_p, n_cur, orig, split ? 2 : 0, out, st);
         if (rc) return rc;
-        if (plan->ok) {
-            if (plan->smem > 48 * 1024)
-                CU_TRY(cudaFuncSetAttribute(belief_tiled_kernel<T, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan->smem));
-            belief_tiled_kernel<T, OUT><<<tiles_cur, h->tb, plan->smem, st>>>(
-                (const NodeMeta*)h->d_nodes.p, (const BeliefGroup*)plan->groups.p, plan->n_groups, pl_p, h->PL,
-                h->tb, h->V, plan->stride, n_cur, d_out, (const uint8_t*)h->d_status.p, (const int32_t*)h->d_sweeps.p,
-                d_out_sweeps, d_out_conv, orig, split ? 2 : 0);
-        } else {
-            belief_kernel<T, OUT><<<tiles, h->tb, 0, st>>>((const NodeMeta*)h->d_nodes.p, h->N, (const T*)h->d_pl.p, h->PL, h->tb,
-                                                        h->V, n, d_out, (const uint8_t*)h->d_status.p,
-                                                        (const int32_t*)h->d_sweeps.p, d_out_sweeps, d_out_conv);
-        }
-        CU_TRY(cudaGetLastError());
-        h->last_kernel_launches++;
     }
-    if (scored) {
-        const int rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 0, d_out_logev, d_out ? nullptr : d_out_sweeps,
-                                       d_out ? nullptr : d_out_conv, st, d_counts, d_weights);
+    if (out.scored()) {
+        const int rc = launch_logev<T>(h, pl_p, msg_p, n_cur, orig, 0, out, st);
         if (rc) return rc;
     }
     if (planned_sweeps) *planned_sweeps = eps_mode ? -1 : (int64_t)total_sweeps * n;
@@ -1106,8 +1134,8 @@ int run_chunk(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_p
 // The whole path for n cases in ONE launch of the on-chip kernel (bnbp_onchip.cuh): init, every sweep, the
 // stopping rule and the beliefs; nothing but evidence in and marginals out touches HBM.
 template <typename T, typename OUT>
-int run_onchip(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out,
-               int32_t* d_out_sweeps, uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps)
+int run_onchip(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, const RunOutputs& out,
+               cudaStream_t st, int64_t* planned_sweeps)
 {
     NvtxRange nvtx_chunk("bnbp: chunk, on-chip kernel (init, every sweep, beliefs in one launch)");
     const bool eps_mode = prm.epsilon > 0.0;
@@ -1124,7 +1152,7 @@ int run_onchip(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_
     a.ev_off = reinterpret_cast<const long long*>(de.ev_off); a.ev_base = de.ev_base;
     a.ev_node = de.ev_node; a.ev_state = de.ev_state;
     a.n_cases = n;
-    a.out = d_out; a.out_sweeps = d_out_sweeps; a.out_conv = d_out_conv;
+    a.out = (OUT*)out.marginals; a.out_sweeps = out.sweeps; a.out_conv = out.converged;
     a.bel_col = (const int*)h->d_belcol.p; a.out_stride = h->Vout;
     a.ticket = ticket; a.error_flag = misc + 1;
     a.eps = (T)prm.epsilon; a.damping = (T)prm.damping;
@@ -1212,23 +1240,20 @@ __global__ void gather_columns_kernel(const OUT* __restrict__ src, OUT* __restri
 // rows into a staging buffer and the asked-for columns are gathered into the output (the on-chip kernel writes
 // only those in the first place).
 template <typename T, typename OUT>
-int run_any(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, OUT* d_out, int32_t* d_out_sweeps,
-            uint8_t* d_out_conv, cudaStream_t st, int64_t* planned_sweeps, double* d_out_logev = nullptr,
-            double* d_counts = nullptr, const double* d_weights = nullptr)
+int run_any(bnbp_handle* h, int64_t n, const DevEvidence& de, const bnbp_run_params& prm, const RunOutputs& out,
+            cudaStream_t st, int64_t* planned_sweeps)
 {
-    if (h->run_onchip) return run_onchip<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps);
-    if (h->q_nodes.empty() || !d_out)
-        return run_chunk<T, OUT>(h, n, de, prm, d_out, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev,
-                                 d_counts, d_weights);
+    if (h->run_onchip) return run_onchip<T, OUT>(h, n, de, prm, out, st, planned_sweeps);
+    if (h->q_nodes.empty() || !out.marginals) return run_chunk<T, OUT>(h, n, de, prm, out, st, planned_sweeps);
     int rc = h->s_full.ensure((size_t)n * h->V * sizeof(OUT));
     if (rc) return rc;
-    if ((rc = run_chunk<T, OUT>(h, n, de, prm, (OUT*)h->s_full.p, d_out_sweeps, d_out_conv, st, planned_sweeps, d_out_logev,
-                                d_counts, d_weights)))
-        return rc;
+    RunOutputs full = out;
+    full.marginals = h->s_full.p;
+    if ((rc = run_chunk<T, OUT>(h, n, de, prm, full, st, planned_sweeps))) return rc;
     const int64_t total = n * h->Vout;
     if (total > 0) {
         gather_columns_kernel<OUT><<<(unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(
-            (const OUT*)h->s_full.p, d_out, n, h->V, h->Vout, (const int32_t*)h->d_colmap.p);
+            (const OUT*)h->s_full.p, (OUT*)out.marginals, n, h->V, h->Vout, (const int32_t*)h->d_colmap.p);
         CU_TRY(cudaGetLastError());
         h->last_kernel_launches++;
     }
@@ -1307,8 +1332,7 @@ int comm_resources(bnbp_handle* h)
     CU_TRY(cudaStreamCreateWithFlags(&h->comm_stream, cudaStreamNonBlocking));
     int rc = h->d_summary.ensure(8 * 8);
     if (rc) return rc;
-    CU_TRY(cudaMallocHost((void**)&h->pin_summary, 8 * 8));
-    return BNBP_OK;
+    return h->pin_summary.ensure(8 * 8);
 }
 
 #define NCCL_TRY(expr)                                                                              \
@@ -1341,16 +1365,17 @@ int enqueue_summary(bnbp_handle* h, const int32_t* d_sweeps, const uint8_t* d_co
 // reported one device's share)
 int fetch_summary(bnbp_handle* h, cudaStream_t st)
 {
-    CU_TRY(cudaMemcpyAsync(h->pin_summary, h->d_summary.p, 8 * 8, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(h->pin_summary.p, h->d_summary.p, 8 * 8, cudaMemcpyDeviceToHost, st));
     return BNBP_OK;
 }
 
 void read_summary(const bnbp_handle* h, bnbp_summary* out)
 {
-    out->case_sweeps = h->pin_summary[0];
-    out->not_converged = h->pin_summary[1];
-    out->n_cases = h->pin_summary[2];
-    out->max_sweeps = h->pin_summary[4];
+    const int64_t* s = (const int64_t*)h->pin_summary.p;
+    out->case_sweeps = s[0];
+    out->not_converged = s[1];
+    out->n_cases = s[2];
+    out->max_sweeps = s[4];
 }
 
 void shard_range(int64_t n, int g, int G, int64_t* lo, int64_t* hi)
@@ -1989,93 +2014,38 @@ int build_layout(const bnbp_flat_network* net, const bnbp_options* opt, bnbp_han
 }
 
 // What the log-evidence and expected-counts calls refuse (before anything is enqueued, so the handle stays usable).
-// counts_call: the expected-counts call, whose counts array must be given and whose out_log_evidence may be NULL.
-int logev_refusal(const bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const double* out_logev,
-                  bool counts_call = false, const double* counts = nullptr)
+// The expected-counts call must be given its counts array; its out_log_evidence may be NULL.
+int logev_refusal(const bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const RunOutputs& out)
 {
-    if (counts_call && !counts) return fail(BNBP_ERR_INVALID, "expected counts: counts is NULL");
-    if (!counts_call && !out_logev) return fail(BNBP_ERR_INVALID, "log-evidence: out_log_evidence is NULL");
-    const std::string what = counts_call ? "expected counts" : "log-evidence";
+    const bool em = out.entry == RunOutputs::EXPECTED_COUNTS;
+    if (em && !out.counts) return fail(BNBP_ERR_INVALID, "expected counts: counts is NULL");
+    if (!em && !out.logev) return fail(BNBP_ERR_INVALID, "log-evidence: out_log_evidence is NULL");
     if (ev->ev_values)
-        return fail(BNBP_ERR_INVALID, what + (counts_call ? " take" : " takes") +
-                                          " hard evidence: soft evidence rows are not an indicator factor");
+        return fail(BNBP_ERR_INVALID, em ? "expected counts take hard evidence: soft evidence rows are not an indicator factor"
+                                         : "log-evidence takes hard evidence: soft evidence rows are not an indicator factor");
     if (prm->semiring == BNBP_MAX_PRODUCT)
-        return fail(BNBP_ERR_INVALID, what + (counts_call ? " are" : " is") + " a sum-product quantity: BNBP_MAX_PRODUCT is refused");
+        return fail(BNBP_ERR_INVALID, em ? "expected counts are a sum-product quantity: BNBP_MAX_PRODUCT is refused"
+                                         : "log-evidence is a sum-product quantity: BNBP_MAX_PRODUCT is refused");
     const bnbp_handle* l = h->members.empty() ? h : h->members[0];
     if (l->TS > 0)
-        return fail(BNBP_ERR_INVALID, what + ": the handle has dense-path nodes; create it with dense_min_cpt = -1");
+        return fail(BNBP_ERR_INVALID, em ? "expected counts: the handle has dense-path nodes; create it with dense_min_cpt = -1"
+                                         : "log-evidence: the handle has dense-path nodes; create it with dense_min_cpt = -1");
     if (prm->gather)
-        return fail(BNBP_ERR_INVALID, what + (counts_call ? ": gather is not supported (the counts stay on this rank)"
-                                                          : ": gather is not supported (the scores stay on this rank)"));
+        return fail(BNBP_ERR_INVALID, em ? "expected counts: gather is not supported (the counts stay on this rank)"
+                                         : "log-evidence: gather is not supported (the scores stay on this rank)");
     return BNBP_OK;
 }
 
-// bnbp_run_batch on a group handle (bnbp_create_multi): contiguous case ranges, one host thread per device, every
-// device copies its rows straight into the caller's buffers; then the convergence summary is all-reduced over the
-// group's communicator (one grouped NCCL call from this thread).
-// counts (expected-counts call): every member adds into its own zeroed host buffer; the buffers are summed in member
-// order and the sum is added into counts.
-int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals, int32_t* out_sweeps,
-              uint8_t* out_converged, double* out_logev, double* counts = nullptr, const double* weights = nullptr)
+// The checks of the evidence batch every run-batch call makes, and the statistics of the last run reset
+int begin_run(bnbp_handle* h, const bnbp_evidence* ev)
 {
     if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
     if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
-    const int G = (int)g->members.size();
-    std::vector<int32_t> q, belcol, colmap;
-    int rc = query_columns(g, *prm, &q, &belcol, &colmap);
-    if (rc) return rc;
-    const size_t row_bytes = colmap.size() * (prm->out_precision == BNBP_OUT_FP32 ? 4 : 8);
-    std::vector<int> rcs((size_t)G, BNBP_OK);
-    std::vector<std::string> errs((size_t)G);
-    std::vector<int64_t> lo((size_t)G), hi((size_t)G);
-    for (int i = 0; i < G; ++i) shard_range(ev->n_cases, i, G, &lo[(size_t)i], &hi[(size_t)i]);
-    std::vector<std::vector<double>> part(counts ? (size_t)G : 0, std::vector<double>((size_t)g->members[0]->cpt_values, 0.0));
-    auto work = [&](int i) {
-        bnbp_evidence e = *ev;
-        e.n_cases = hi[(size_t)i] - lo[(size_t)i];
-        e.ev_off = ev->ev_off ? ev->ev_off + lo[(size_t)i] : nullptr;
-        void* const marg = out_marginals ? (char*)out_marginals + (size_t)lo[(size_t)i] * row_bytes : nullptr;
-        int32_t* const sw = out_sweeps ? out_sweeps + lo[(size_t)i] : nullptr;
-        uint8_t* const cv = out_converged ? out_converged + lo[(size_t)i] : nullptr;
-        double* const lev = out_logev ? out_logev + lo[(size_t)i] : nullptr;
-        if (counts)
-            rcs[(size_t)i] = bnbp_run_batch_expected_counts(g->members[(size_t)i], &e, prm, weights ? weights + lo[(size_t)i] : nullptr,
-                                                            part[(size_t)i].data(), marg, sw, cv, lev);
-        else
-            rcs[(size_t)i] = out_logev ? bnbp_run_batch_log_evidence(g->members[(size_t)i], &e, prm, marg, sw, cv, lev)
-                                       : bnbp_run_batch(g->members[(size_t)i], &e, prm, marg, sw, cv);
-        if (rcs[(size_t)i]) errs[(size_t)i] = bnbp_last_error();      // the error channel is thread-local
-    };
-    std::vector<std::thread> threads;
-    for (int i = 1; i < G; ++i) threads.emplace_back(work, i);
-    work(0);
-    for (std::thread& t : threads) t.join();
-    for (int i = 0; i < G; ++i)
-        if (rcs[(size_t)i]) return fail(rcs[(size_t)i], "device " + std::to_string(g->members[(size_t)i]->device) + ": " + errs[(size_t)i]);
-    if (counts) {
-        for (int i = 1; i < G; ++i)
-            for (size_t j = 0; j < part[0].size(); ++j) part[0][j] += part[(size_t)i][j];
-        for (size_t j = 0; j < part[0].size(); ++j) counts[j] += part[0][j];
-    }
-    // summary: per-case counts are still on each device (whole-shard staging of bnbp_run_batch)
-    NCCL_TRY(NCCL(GroupStart)());
-    for (int i = 0; i < G; ++i) {
-        bnbp_handle* m = g->members[(size_t)i];
-        CU_TRY(cudaSetDevice(m->device));
-        const int64_t n = hi[(size_t)i] - lo[(size_t)i];
-        if ((rc = enqueue_summary(m, (const int32_t*)m->s_out_sweeps.p, (const uint8_t*)m->s_out_conv.p, n, m->stream))) {
-            NCCL(GroupEnd)();
-            return rc;
-        }
-    }
-    NCCL_TRY(NCCL(GroupEnd)());
-    for (int i = 0; i < G; ++i) {
-        CU_TRY(cudaSetDevice(g->members[(size_t)i]->device));
-        if ((rc = fetch_summary(g->members[(size_t)i], g->members[(size_t)i]->stream))) return rc;
-        CU_TRY(wait_stream(g->members[(size_t)i]->stream));
-    }
-    read_summary(g->members[0], &g->last_summary);
-    g->last_case_sweeps = g->last_summary.case_sweeps;
+    h->last_sweep_launches = h->last_kernel_launches = h->last_dense_launches = h->last_dense_tc_launches = 0;
+    h->last_case_sweeps = 0;
+    h->ev_sweep_used = 0;
+    h->ev_dense_used = 0;
+    h->last_compactions = 0;
     return BNBP_OK;
 }
 
@@ -2189,17 +2159,7 @@ void bnbp_destroy(bnbp_handle* h)
     if (h->comm) { if (h->stream) cudaStreamSynchronize(h->stream); NCCL(CommAbort)(h->comm); h->comm = nullptr; }
     if (h->comm_stream) { cudaStreamSynchronize(h->comm_stream); cudaStreamDestroy(h->comm_stream); }
     for (cudaEvent_t e : h->ev_comm) cudaEventDestroy(e);
-    if (h->pin_summary) cudaFreeHost(h->pin_summary);
-    for (DevBuf* b : {&h->d_belcol, &h->d_colmap, &h->s_full, &h->d_summary}) b->release();
     if (h->stream) cudaStreamSynchronize(h->stream);
-    for (DevBuf* b : {&h->d_nodes, &h->d_e_card, &h->d_e_lam_out, &h->d_c_pi_out, &h->d_cpt, &h->d_pl_init, &h->d_pl,
-                      &h->d_msg[0], &h->d_msg[1], &h->d_evbits, &h->d_delta, &h->d_status, &h->d_sweeps, &h->d_misc,
-                      &h->d_pl2, &h->d_msg2[0], &h->d_msg2[1], &h->d_evbits2, &h->d_orig[0], &h->d_orig[1], &h->d_src_pos, &h->d_tile_count,
-                      &h->d_evst, &h->d_lw_order, &h->d_lw_par, &h->d_lw_cpt, &h->d_lw_out, &h->d_lw_wsum, &h->d_djobs, &h->d_dytab, &h->d_ddig, &h->d_cpt_t, &h->d_tscr,
-                      &h->s_ev_off, &h->s_ev_node, &h->s_ev_state, &h->s_ev_val_off, &h->s_ev_values, &h->s_out[0], &h->s_out[1], &h->s_out_all,
-                      &h->s_out_sweeps, &h->s_out_conv, &h->s_out_logev, &h->s_counts, &h->s_weights})
-        b->release();
-    for (auto& kv : h->belief_plans) kv.second.groups.release();
     for (cudaEvent_t e : h->ev_chunk) cudaEventDestroy(e);
     if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
     if (h->h2d_stream) { cudaStreamSynchronize(h->h2d_stream); cudaStreamDestroy(h->h2d_stream); }
@@ -2212,11 +2172,8 @@ void bnbp_destroy(bnbp_handle* h)
         if (h->ev_poll[i]) cudaEventDestroy(h->ev_poll[i]);
     }
     if (h->pinned_poll) cudaFreeHost(h->pinned_poll);
-    if (h->pin_counts) cudaFreeHost(h->pin_counts);
-    if (h->pin_logev) cudaFreeHost(h->pin_logev);
-    if (h->pin_cnt) cudaFreeHost(h->pin_cnt);
     if (h->stream) cudaStreamDestroy(h->stream);
-    delete h;
+    delete h;                             // the device and pinned buffers free themselves, on the handle's device
 }
 
 int bnbp_refresh_cpt(bnbp_handle* h, const double* cpt, int64_t n_values)
@@ -2321,30 +2278,21 @@ int bnbp_spec_source(const bnbp_flat_network* net, const bnbp_options* opt, int3
     return BNBP_OK;
 }
 
-// counts_call: bnbp_run_batch_device_expected_counts (counts / weights are device memory; counts is added into by the
-// scoring launches directly).
-static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
-                            int32_t* out_sweeps, uint8_t* out_converged, double* out_logev, void* stream,
-                            bool counts_call = false, double* counts = nullptr, const double* weights = nullptr)
+// The device-buffer calls: every array of out is device memory (counts is added into by the scoring launches directly)
+static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const RunOutputs& out,
+                            void* stream)
 {
     NvtxRange nvtx_call("bnbp_run_batch_device");
     int rc = validate_params(prm);
     if (rc) return rc;
-    if ((out_logev || counts_call) && (rc = logev_refusal(h, ev, prm, out_logev, counts_call, counts))) return rc;
-    if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
-    if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
+    if (out.scored() && (rc = logev_refusal(h, ev, prm, out))) return rc;
+    if ((rc = begin_run(h, ev))) return rc;
     CU_TRY(cudaSetDevice(h->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-    h->last_sweep_launches = h->last_kernel_launches = h->last_dense_launches = h->last_dense_tc_launches = 0;
-    h->last_case_sweeps = 0;
-    h->ev_sweep_used = 0;
-    h->ev_dense_used = 0;
-    h->last_compactions = 0;
     if (ev->n_cases == 0) return BNBP_OK;
     if (!h->members.empty()) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device: a group handle takes host buffers (bnbp_run_batch); the device path belongs to one device");
     if ((rc = set_query(h, *prm))) return rc;
-    if ((rc = choose_kernels(h, ev->n_cases, *prm, ev->ev_values != nullptr, h->precision != BNBP_FP32,
-                             out_logev != nullptr || counts_call))) return rc;
+    if ((rc = choose_kernels(h, ev->n_cases, *prm, ev->ev_values != nullptr, h->precision != BNBP_FP32, out.scored()))) return rc;
     if (!h->run_onchip && (rc = ensure_state(h, ev->n_cases))) return rc;
     // a flag left by an earlier (unchecked, asynchronous) run must not fail this one
     CU_TRY(cudaMemsetAsync(reinterpret_cast<int32_t*>(h->d_misc.p) + 1, 0, 4, st));
@@ -2363,8 +2311,9 @@ static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_
         h->reserve_sms = std::min(32, 8 * (h->comm_world - 1));
         if (const char* e = getenv("BNBP_GATHER_SMS")) h->reserve_sms = std::max(0, atoi(e));
     }
-    char* const base = (char*)out_marginals;
-    char* const mine = base + (gather ? (size_t)h->comm_rank * (size_t)ev->n_cases * row_bytes : 0);
+    char* const base = (char*)out.marginals;
+    RunOutputs mine = out;                                                // this rank's rows of out.marginals
+    if (gather && base) mine.marginals = base + (size_t)h->comm_rank * (size_t)ev->n_cases * row_bytes;
     int64_t step_cases = h->run_onchip ? ev->n_cases : h->cap;            // on chip: no resident state arena, one launch
     if (exchange) {
         // 8 chunks of >= 8 MB each when the batch allows it: the exchange of chunk i hides behind the kernels of chunk
@@ -2379,15 +2328,9 @@ static int run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_
         const int64_t n = std::min<int64_t>(step_cases, ev->n_cases - c0);
         DevEvidence de{ev->ev_off + c0, 0, ev->ev_node, ev->ev_state, ev->ev_val_off, ev->ev_values, 0};
         int64_t planned = 0;
-        char* const dst = out_marginals ? mine + (size_t)c0 * row_bytes : nullptr;
-        double* const lev = out_logev ? out_logev + c0 : nullptr;
-        const double* const wts = weights ? weights + c0 : nullptr;
-        if (h->precision == BNBP_FP32)
-            rc = run_any<float, float>(h, n, de, *prm, (float*)dst, out_sweeps ? out_sweeps + c0 : nullptr,
-                                       out_converged ? out_converged + c0 : nullptr, st, &planned, lev, counts, wts);
-        else
-            rc = run_any<double, double>(h, n, de, *prm, (double*)dst, out_sweeps ? out_sweeps + c0 : nullptr,
-                                         out_converged ? out_converged + c0 : nullptr, st, &planned, lev, counts, wts);
+        const RunOutputs o = mine.at(c0, row_bytes);
+        rc = h->precision == BNBP_FP32 ? run_any<float, float>(h, n, de, *prm, o, st, &planned)
+                                       : run_any<double, double>(h, n, de, *prm, o, st, &planned);
         if (rc) return rc;
         if (planned < 0) exact = false; else h->last_case_sweeps += planned;
         if (exchange) {
@@ -2431,14 +2374,14 @@ int bnbp_run_batch_device(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
                           int32_t* out_sweeps, uint8_t* out_converged, void* stream)
 {
     if (!h || !ev || !out_marginals) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device: NULL argument");
-    return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, nullptr, stream);
+    return run_batch_device(h, ev, prm, {RunOutputs::PLAIN, out_marginals, out_sweeps, out_converged}, stream);
 }
 
 int bnbp_run_batch_device_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
                                        int32_t* out_sweeps, uint8_t* out_converged, double* out_log_evidence, void* stream)
 {
     if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device_log_evidence: NULL argument");
-    return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, stream);
+    return run_batch_device(h, ev, prm, {RunOutputs::LOG_EVIDENCE, out_marginals, out_sweeps, out_converged, out_log_evidence}, stream);
 }
 
 int bnbp_run_batch_device_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
@@ -2446,8 +2389,8 @@ int bnbp_run_batch_device_expected_counts(bnbp_handle* h, const bnbp_evidence* e
                                           int32_t* out_sweeps, uint8_t* out_converged, double* out_log_evidence, void* stream)
 {
     if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_device_expected_counts: NULL argument");
-    return run_batch_device(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, stream, true, counts,
-                            case_weights);
+    return run_batch_device(h, ev, prm, {RunOutputs::EXPECTED_COUNTS, out_marginals, out_sweeps, out_converged, out_log_evidence,
+                                         counts, case_weights}, stream);
 }
 
 int bnbp_check_errors(bnbp_handle* h, void* stream)
@@ -2458,30 +2401,86 @@ int bnbp_check_errors(bnbp_handle* h, void* stream)
     return check_error_flag(h, stream ? (cudaStream_t)stream : h->stream);
 }
 
-// counts_call: bnbp_run_batch_expected_counts.  The scoring launches add into the handle's zeroed device count arena;
-// it comes back through pinned staging and is added into counts once every chunk has run.
-static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals_v,
-                          int32_t* out_sweeps, uint8_t* out_converged, double* out_logev, bool counts_call = false,
-                          double* counts = nullptr, const double* weights = nullptr)
+static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const RunOutputs& out);
+
+// The host-buffer call on a group handle (bnbp_create_multi): contiguous case ranges, one host thread per device, every
+// device copies its rows straight into the caller's buffers; then the convergence summary is all-reduced over the
+// group's communicator (one grouped NCCL call from this thread).
+// Expected counts: every member adds into its own zeroed host buffer; the buffers are summed in member order and the
+// sum is added into out.counts.
+static int run_group(bnbp_handle* g, const bnbp_evidence* ev, const bnbp_run_params* prm, const RunOutputs& out)
+{
+    const int G = (int)g->members.size();
+    std::vector<int32_t> q, belcol, colmap;
+    int rc = query_columns(g, *prm, &q, &belcol, &colmap);
+    if (rc) return rc;
+    const size_t row_bytes = colmap.size() * (prm->out_precision == BNBP_OUT_FP32 ? 4 : 8);
+    std::vector<int> rcs((size_t)G, BNBP_OK);
+    std::vector<std::string> errs((size_t)G);
+    std::vector<int64_t> lo((size_t)G), hi((size_t)G);
+    for (int i = 0; i < G; ++i) shard_range(ev->n_cases, i, G, &lo[(size_t)i], &hi[(size_t)i]);
+    std::vector<std::vector<double>> part(out.counts ? (size_t)G : 0, std::vector<double>((size_t)g->members[0]->cpt_values, 0.0));
+    auto work = [&](int i) {
+        bnbp_evidence e = *ev;
+        e.n_cases = hi[(size_t)i] - lo[(size_t)i];
+        e.ev_off = ev->ev_off ? ev->ev_off + lo[(size_t)i] : nullptr;
+        RunOutputs o = out.at(lo[(size_t)i], row_bytes);
+        if (out.counts) o.counts = part[(size_t)i].data();
+        rcs[(size_t)i] = run_batch_host(g->members[(size_t)i], &e, prm, o);
+        if (rcs[(size_t)i]) errs[(size_t)i] = bnbp_last_error();      // the error channel is thread-local
+    };
+    std::vector<std::thread> threads;
+    for (int i = 1; i < G; ++i) threads.emplace_back(work, i);
+    work(0);
+    for (std::thread& t : threads) t.join();
+    for (int i = 0; i < G; ++i)
+        if (rcs[(size_t)i]) return fail(rcs[(size_t)i], "device " + std::to_string(g->members[(size_t)i]->device) + ": " + errs[(size_t)i]);
+    if (out.counts) {
+        for (int i = 1; i < G; ++i)
+            for (size_t j = 0; j < part[0].size(); ++j) part[0][j] += part[(size_t)i][j];
+        for (size_t j = 0; j < part[0].size(); ++j) out.counts[j] += part[0][j];
+    }
+    // summary: per-case counts are still on each device (whole-shard staging of bnbp_run_batch)
+    NCCL_TRY(NCCL(GroupStart)());
+    for (int i = 0; i < G; ++i) {
+        bnbp_handle* m = g->members[(size_t)i];
+        CU_TRY(cudaSetDevice(m->device));
+        const int64_t n = hi[(size_t)i] - lo[(size_t)i];
+        if ((rc = enqueue_summary(m, (const int32_t*)m->s_out_sweeps.p, (const uint8_t*)m->s_out_conv.p, n, m->stream))) {
+            NCCL(GroupEnd)();
+            return rc;
+        }
+    }
+    NCCL_TRY(NCCL(GroupEnd)());
+    for (int i = 0; i < G; ++i) {
+        CU_TRY(cudaSetDevice(g->members[(size_t)i]->device));
+        if ((rc = fetch_summary(g->members[(size_t)i], g->members[(size_t)i]->stream))) return rc;
+        CU_TRY(wait_stream(g->members[(size_t)i]->stream));
+    }
+    read_summary(g->members[0], &g->last_summary);
+    g->last_case_sweeps = g->last_summary.case_sweeps;
+    return BNBP_OK;
+}
+
+// The host-buffer calls.  Expected counts: the scoring launches add into the handle's zeroed device count arena; it
+// comes back through pinned staging and is added into out.counts once every chunk has run.
+static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, const RunOutputs& out)
 {
     const auto t_entry = std::chrono::steady_clock::now();
     NvtxRange nvtx_call("bnbp_run_batch (host buffers: H2D evidence | kernels | D2H marginals, pipelined by chunk)");
     int rc = validate_params(prm);
     if (rc) return rc;
-    if ((out_logev || counts_call) && (rc = logev_refusal(h, ev, prm, out_logev, counts_call, counts))) return rc;
-    if (counts_call && weights && ev->n_cases > 0)
+    if (out.scored() && (rc = logev_refusal(h, ev, prm, out))) return rc;
+    if (out.weights && ev->n_cases > 0)
         for (int64_t c = 0; c < ev->n_cases; ++c)
-            if (!(std::isfinite(weights[c]) && weights[c] >= 0.0))
+            if (!(std::isfinite(out.weights[c]) && out.weights[c] >= 0.0))
                 return fail(BNBP_ERR_INVALID, "expected counts: case_weights[" + std::to_string(c) + "] is not finite and >= 0");
-    if (!h->members.empty())
-        return run_group(h, ev, prm, out_marginals_v, out_sweeps, out_converged, out_logev, counts_call ? counts : nullptr, weights);
+    if ((rc = begin_run(h, ev))) return rc;
+    if (!h->members.empty()) return run_group(h, ev, prm, out);
     const bool out_f32 = prm->out_precision == BNBP_OUT_FP32;
     if (out_f32 && h->precision != BNBP_FP32)
         return fail(BNBP_ERR_INVALID, "out_precision FP32 needs an fp32 handle (an fp64 handle returns the reference's doubles)");
     if (prm->out_precision < BNBP_OUT_DEFAULT || prm->out_precision > BNBP_OUT_FP32) return fail(BNBP_ERR_INVALID, "out_precision out of range");
-    char* const out_marginals = (char*)out_marginals_v;
-    if (ev->n_cases < 0) return fail(BNBP_ERR_INVALID, "n_cases < 0");
-    if (ev->n_cases > 0 && !ev->ev_off) return fail(BNBP_ERR_INVALID, "ev_off is NULL");
     const int64_t nnz = ev->n_cases ? ev->ev_off[ev->n_cases] : 0;
     if (nnz > 0 && !ev->ev_node) return fail(BNBP_ERR_INVALID, "ev_node is NULL");
     const bool soft = ev->ev_values != nullptr;
@@ -2492,15 +2491,10 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     // (the per-case monotonicity check runs chunk by chunk below, while the device works on the chunk before)
     CU_TRY(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    h->last_sweep_launches = h->last_kernel_launches = h->last_dense_launches = h->last_dense_tc_launches = 0;
-    h->last_case_sweeps = 0;
-    h->ev_sweep_used = 0;
-    h->ev_dense_used = 0;
-    h->last_compactions = 0;
     if (ev->n_cases == 0) return BNBP_OK;
     h->reserve_sms = 0;
     if ((rc = set_query(h, *prm))) return rc;
-    if ((rc = choose_kernels(h, ev->n_cases, *prm, soft, !out_f32, out_logev != nullptr || counts_call))) return rc;
+    if ((rc = choose_kernels(h, ev->n_cases, *prm, soft, !out_f32, out.scored()))) return rc;
     if ((rc = measure_rates(h))) return rc;
     // Chunk pipeline on three streams: evidence of chunk i+1 goes up (h2d_stream) and the marginals of
     // chunk i-1 come down (copy_stream) while init/sweeps/beliefs of chunk i run.  Marginals are 8*V
@@ -2542,7 +2536,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     // else a ring of two chunk-sized slots.
     const size_t row_bytes = (size_t)h->Vout * out_elem;
     bool whole = (size_t)ev->n_cases * row_bytes <= h->s_out_all.bytes;
-    if (!out_marginals) whole = true;                     // no marginals asked (log-evidence only): nothing to stage
+    if (!out.marginals) whole = true;                     // no marginals asked (log-evidence only): nothing to stage
     if (!whole && !getenv("BNBP_STAGING_RING")) {
         size_t free_b = 0, total_b = 0;
         CU_TRY(cudaMemGetInfo(&free_b, &total_b));
@@ -2559,31 +2553,29 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     // pageable, and a pageable D2H per chunk would block the host and serialise the pipeline
     if ((rc = h->s_out_sweeps.ensure((size_t)ev->n_cases * 4))) return rc;
     if ((rc = h->s_out_conv.ensure((size_t)ev->n_cases))) return rc;
-    if (h->pin_counts_bytes < (size_t)ev->n_cases * 5) {
-        if (h->pin_counts) cudaFreeHost(h->pin_counts);
-        h->pin_counts = nullptr;
-        h->pin_counts_bytes = 0;
-        CU_TRY(cudaMallocHost(&h->pin_counts, (size_t)ev->n_cases * 5));
-        h->pin_counts_bytes = (size_t)ev->n_cases * 5;
-    }
-    int32_t* const pin_sweeps = (int32_t*)h->pin_counts;
-    uint8_t* const pin_conv = (uint8_t*)h->pin_counts + (size_t)ev->n_cases * 4;
-    if (out_logev) {
+    if ((rc = h->pin_counts.ensure((size_t)ev->n_cases * 5))) return rc;
+    if (out.logev) {
         if ((rc = h->s_out_logev.ensure((size_t)ev->n_cases * 8))) return rc;
-        if (h->pin_logev_bytes < (size_t)ev->n_cases * 8) {
-            if (h->pin_logev) cudaFreeHost(h->pin_logev);
-            h->pin_logev = nullptr;
-            h->pin_logev_bytes = 0;
-            CU_TRY(cudaMallocHost((void**)&h->pin_logev, (size_t)ev->n_cases * 8));
-            h->pin_logev_bytes = (size_t)ev->n_cases * 8;
-        }
+        if ((rc = h->pin_logev.ensure((size_t)ev->n_cases * 8))) return rc;
     }
     const size_t count_bytes = std::max<size_t>(16, (size_t)h->cpt_values * 8);
-    if (counts_call) {
+    if (out.counts) {
         if ((rc = h->s_counts.ensure(count_bytes))) return rc;
-        if (!h->pin_cnt) CU_TRY(cudaMallocHost((void**)&h->pin_cnt, count_bytes));
-        if (weights && (rc = h->s_weights.ensure((size_t)ev->n_cases * 8))) return rc;
+        if ((rc = h->pin_cnt.ensure(count_bytes))) return rc;
+        if (out.weights && (rc = h->s_weights.ensure((size_t)ev->n_cases * 8))) return rc;
     }
+    int32_t* const pin_sweeps = (int32_t*)h->pin_counts.p;
+    uint8_t* const pin_conv = (uint8_t*)h->pin_counts.p + (size_t)ev->n_cases * 4;
+    double* const pin_logev = (double*)h->pin_logev.p;
+    double* const pin_cnt = (double*)h->pin_cnt.p;
+    // the same outputs staged on the device (marginals: the whole batch, or the ring slot of each chunk below)
+    RunOutputs staged = out;
+    staged.marginals = out.marginals && whole ? h->s_out_all.p : nullptr;
+    staged.sweeps = (int32_t*)h->s_out_sweeps.p;
+    staged.converged = (uint8_t*)h->s_out_conv.p;
+    if (out.logev) staged.logev = (double*)h->s_out_logev.p;
+    if (out.counts) staged.counts = (double*)h->s_counts.p;
+    if (out.weights) staged.weights = (const double*)h->s_weights.p;
     // evidence staging for the whole batch (absolute offsets, like bnbp_run_batch_device)
     if ((rc = h->s_ev_off.ensure((size_t)(ev->n_cases + 1) * 8))) return rc;
     if ((rc = h->s_ev_node.ensure(std::max<size_t>(16, (size_t)nnz * 4)))) return rc;
@@ -2612,7 +2604,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
         fprintf(stderr, "\n");
     }
     CU_TRY(cudaMemsetAsync(reinterpret_cast<int32_t*>(h->d_misc.p) + 1, 0, 4, st));
-    if (counts_call) CU_TRY(cudaMemsetAsync(h->s_counts.p, 0, count_bytes, st));
+    if (out.counts) CU_TRY(cudaMemsetAsync(h->s_counts.p, 0, count_bytes, st));
     cudaStream_t cs = h->copy_stream, hs = h->h2d_stream;
     struct Drain {                       // no path leaves this call with copies from/to host memory in flight
         cudaStream_t a, b, c;
@@ -2620,8 +2612,8 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     } drain{hs, st, cs};
     CU_TRY(cudaEventRecord(h->ev_total[0], st));
     CU_TRY(cudaStreamWaitEvent(hs, h->ev_total[0], 0));   // uploads start with the call on the device timeline
-    if (counts_call && weights)                            // ahead of every chunk's evidence: each chunk waits for those
-        CU_TRY(cudaMemcpyAsync(h->s_weights.p, weights, (size_t)ev->n_cases * 8, cudaMemcpyHostToDevice, hs));
+    if (out.weights)                                       // ahead of every chunk's evidence: each chunk waits for those
+        CU_TRY(cudaMemcpyAsync(h->s_weights.p, out.weights, (size_t)ev->n_cases * 8, cudaMemcpyHostToDevice, hs));
     std::vector<cudaEvent_t> tev;                     // BNBP_TRACE: device timeline of the pipeline
     auto mark = [&](cudaStream_t s) {
         if (!trace) return;
@@ -2674,35 +2666,28 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
         CU_TRY(cudaEventRecord(e_up, hs));
         nvtx_h2d.reset();
         CU_TRY(cudaStreamWaitEvent(st, e_up, 0));
-        char* slot = !out_marginals ? nullptr : whole ? (char*)h->s_out_all.p + (size_t)c0 * row_bytes : (char*)h->s_out[idx & 1].p;
-        double* const lev = out_logev ? (double*)h->s_out_logev.p + c0 : nullptr;
-        double* const cnt = counts_call ? (double*)h->s_counts.p : nullptr;
-        const double* const wts = counts_call && weights ? (const double*)h->s_weights.p + c0 : nullptr;
+        RunOutputs o = staged.at(c0, row_bytes);
+        if (!whole) o.marginals = h->s_out[idx & 1].p;
         if (!whole && idx >= 2) CU_TRY(cudaStreamWaitEvent(st, h->ev_chunk[3 * (idx - 2) + 2], 0));   // ring slot is free again
         stamp("enqueue chunk", idx);
         mark(st);
-        if (h->precision == BNBP_FP32 && out_f32)
-            rc = run_any<float, float>(h, n, de, *prm, (float*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev, cnt, wts);
-        else if (h->precision == BNBP_FP32)
-            rc = run_any<float, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev, cnt, wts);
-        else
-            rc = run_any<double, double>(h, n, de, *prm, (double*)slot, (int32_t*)h->s_out_sweeps.p + c0, (uint8_t*)h->s_out_conv.p + c0, st, nullptr, lev, cnt, wts);
+        if (h->precision == BNBP_FP32 && out_f32) rc = run_any<float, float>(h, n, de, *prm, o, st, nullptr);
+        else if (h->precision == BNBP_FP32) rc = run_any<float, double>(h, n, de, *prm, o, st, nullptr);
+        else rc = run_any<double, double>(h, n, de, *prm, o, st, nullptr);
         if (rc) return rc;
         mark(st);
         CU_TRY(cudaEventRecord(e_done, st));
         CU_TRY(cudaStreamWaitEvent(cs, e_done, 0));
         mark(cs);
         NvtxRange nvtx_d2h("bnbp: enqueue D2H marginals of a chunk");
-        if (out_marginals)
-            CU_TRY(cudaMemcpyAsync(out_marginals + (size_t)c0 * row_bytes, slot, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, cs));
-        if (out_logev) CU_TRY(cudaMemcpyAsync(h->pin_logev + c0, lev, (size_t)n * 8, cudaMemcpyDeviceToHost, cs));
+        if (out.marginals)
+            CU_TRY(cudaMemcpyAsync((char*)out.marginals + (size_t)c0 * row_bytes, o.marginals, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, cs));
+        if (out.logev) CU_TRY(cudaMemcpyAsync(pin_logev + c0, o.logev, (size_t)n * 8, cudaMemcpyDeviceToHost, cs));
         mark(cs);
         // per-case counts: into the library's pinned staging (the caller's arrays are usually pageable, and
         // a pageable D2H would block this thread until the chunk is done)
-        if (out_sweeps)
-            CU_TRY(cudaMemcpyAsync(pin_sweeps + c0, (const int32_t*)h->s_out_sweeps.p + c0, (size_t)n * 4, cudaMemcpyDeviceToHost, cs));
-        if (out_converged)
-            CU_TRY(cudaMemcpyAsync(pin_conv + c0, (const uint8_t*)h->s_out_conv.p + c0, (size_t)n, cudaMemcpyDeviceToHost, cs));
+        if (out.sweeps) CU_TRY(cudaMemcpyAsync(pin_sweeps + c0, o.sweeps, (size_t)n * 4, cudaMemcpyDeviceToHost, cs));
+        if (out.converged) CU_TRY(cudaMemcpyAsync(pin_conv + c0, o.converged, (size_t)n, cudaMemcpyDeviceToHost, cs));
         CU_TRY(cudaEventRecord(e_copied, cs));
         stamp("enqueued copy", idx);
     }
@@ -2710,7 +2695,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     // copy_stream is in order: everything before e_last has left when it fires
     stamp("all enqueued", idx);
     // the call returns with every result on the host
-    if (counts_call) CU_TRY(cudaMemcpyAsync(h->pin_cnt, h->s_counts.p, count_bytes, cudaMemcpyDeviceToHost, st));
+    if (out.counts) CU_TRY(cudaMemcpyAsync(pin_cnt, h->s_counts.p, count_bytes, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamWaitEvent(st, e_last, 0));
     CU_TRY(cudaEventRecord(h->ev_total[1], st));
     h->total_recorded = true;
@@ -2718,7 +2703,7 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
     NvtxRange nvtx_wait("bnbp: wait for the streams");
     if ((rc = check_error_flag(h, st))) return rc;
     CU_TRY(wait_stream(cs));
-    if (counts_call) CU_TRY(wait_stream(st));
+    if (out.counts) CU_TRY(wait_stream(st));
     h->last_host_wait_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_wait).count();
     stamp("done", idx);
     for (size_t i = 0; i + 3 < tev.size(); i += 4) {
@@ -2730,16 +2715,16 @@ static int run_batch_host(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_ru
         fprintf(stderr, "[bnbp] chunk %zu: compute %.3f..%.3f ms, copy %.3f..%.3f ms (device timeline)\n", i / 4, a, b, c, d);
     }
     for (cudaEvent_t e : tev) cudaEventDestroy(e);
-    if (out_sweeps) memcpy(out_sweeps, pin_sweeps, (size_t)ev->n_cases * 4);
-    if (out_converged) memcpy(out_converged, pin_conv, (size_t)ev->n_cases);
-    if (out_logev) memcpy(out_logev, h->pin_logev, (size_t)ev->n_cases * 8);
-    if (counts_call)
-        for (int64_t j = 0; j < h->cpt_values; ++j) counts[j] += h->pin_cnt[j];
+    if (out.sweeps) memcpy(out.sweeps, pin_sweeps, (size_t)ev->n_cases * 4);
+    if (out.converged) memcpy(out.converged, pin_conv, (size_t)ev->n_cases);
+    if (out.logev) memcpy(out.logev, pin_logev, (size_t)ev->n_cases * 8);
+    if (out.counts)
+        for (int64_t j = 0; j < h->cpt_values; ++j) out.counts[j] += pin_cnt[j];
     if (!(prm->epsilon > 0.0)) {
         h->last_case_sweeps = ev->n_cases * (int64_t)prm->max_sweeps;     // fixed count: every case ran them all
-    } else if (out_sweeps) {
+    } else if (out.sweeps) {
         int64_t s = 0;
-        for (int64_t c = 0; c < ev->n_cases; ++c) s += out_sweeps[c];
+        for (int64_t c = 0; c < ev->n_cases; ++c) s += out.sweeps[c];
         h->last_case_sweeps = s;
     } else {
         h->last_case_sweeps = -1;
@@ -2752,14 +2737,14 @@ int bnbp_run_batch(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_param
                    int32_t* out_sweeps, uint8_t* out_converged)
 {
     if (!h || !ev || !out_marginals) return fail(BNBP_ERR_INVALID, "bnbp_run_batch: NULL argument");
-    return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, nullptr);
+    return run_batch_host(h, ev, prm, {RunOutputs::PLAIN, out_marginals, out_sweeps, out_converged});
 }
 
 int bnbp_run_batch_log_evidence(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm, void* out_marginals,
                                 int32_t* out_sweeps, uint8_t* out_converged, double* out_log_evidence)
 {
     if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_log_evidence: NULL argument");
-    return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence);
+    return run_batch_host(h, ev, prm, {RunOutputs::LOG_EVIDENCE, out_marginals, out_sweeps, out_converged, out_log_evidence});
 }
 
 int bnbp_run_batch_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, const bnbp_run_params* prm,
@@ -2767,7 +2752,8 @@ int bnbp_run_batch_expected_counts(bnbp_handle* h, const bnbp_evidence* ev, cons
                                    uint8_t* out_converged, double* out_log_evidence)
 {
     if (!h || !ev || !prm) return fail(BNBP_ERR_INVALID, "bnbp_run_batch_expected_counts: NULL argument");
-    return run_batch_host(h, ev, prm, out_marginals, out_sweeps, out_converged, out_log_evidence, true, counts, case_weights);
+    return run_batch_host(h, ev, prm, {RunOutputs::EXPECTED_COUNTS, out_marginals, out_sweeps, out_converged, out_log_evidence,
+                                       counts, case_weights});
 }
 
 int bnbp_lw_run_batch(bnbp_handle* h, const bnbp_evidence* ev, int64_t n_samples, uint64_t seed, double* out_marginals,
@@ -2894,8 +2880,6 @@ int bnbp_estimate_cpt(const bnbp_flat_network* net, const int32_t* samples, cons
     }
     if (device >= 0) CU_TRY(cudaSetDevice(device));
     DevBuf d_nodes, d_par, d_rows, d_samples, d_mult, d_counts, d_cpt, d_flag;
-    struct Free { std::vector<DevBuf*> b; ~Free() { for (DevBuf* x : b) x->release(); } }
-        guard{{&d_nodes, &d_par, &d_rows, &d_samples, &d_mult, &d_counts, &d_cpt, &d_flag}};
     int rc;
     if ((rc = d_nodes.ensure(nodes.size() * sizeof(NodeMeta)))) return rc;
     if ((rc = d_par.ensure(std::max<size_t>(16, (size_t)E * 4)))) return rc;

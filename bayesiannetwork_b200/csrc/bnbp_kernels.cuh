@@ -235,35 +235,9 @@ __global__ void finalize_kernel(uint8_t* status, int32_t* sweeps, const T* delta
     }
 }
 
-// K4: belief = normalize(pi .* lambda) (:151-158), written case-major [case][sum r].
-template <typename T, typename OUT>
-__global__ void __launch_bounds__(512)
-belief_kernel(const NodeMeta* nodes, int n_nodes, const T* pl_all, int PL, int TBi, int V,
-              int64_t n_valid, OUT* out, const uint8_t* status, const int32_t* sweeps,
-              int32_t* out_sweeps, uint8_t* out_conv)
-{
-    const int tile = blockIdx.x, lane = threadIdx.x;
-    const size_t TB = (size_t)TBi;
-    const int64_t c = (int64_t)tile * TBi + lane;
-    if (c >= n_valid) return;
-    const T* pl = pl_all + ((size_t)tile * PL) * TB + lane;
-    OUT* o = out + (size_t)c * V;
-    for (int X = 0; X < n_nodes; ++X) {
-        const NodeMeta nd = nodes[X];
-        const int r = nd.card;
-        T s = T(0);
-        for (int x = 0; x < r; ++x)
-            s = fma(pl[(size_t)(nd.pl_off + x) * TB], pl[(size_t)(nd.pl_off + r + x) * TB], s);
-        for (int x = 0; x < r; ++x)
-            o[nd.bel_off + x] = (OUT)(mul_rn(pl[(size_t)(nd.pl_off + x) * TB], pl[(size_t)(nd.pl_off + r + x) * TB]) / s);
-    }
-    if (out_sweeps) out_sweeps[c] = sweeps[c];
-    if (out_conv) out_conv[c] = status[c];
-}
-
-// K4, tiled: the same belief (:151-158), but the case-major rows leave through shared memory so that
-// global stores are coalesced.  belief_kernel above lets every thread write its own 8*V-byte row
-// (32 rows per warp store = 32 sectors with 8 valid bytes each).  Here every WARP owns 32 cases and
+// K4: belief = normalize(pi .* lambda) (:151-158), written case-major [case][sum r].  The rows leave
+// through shared memory so that global stores are coalesced: a thread writing its own 8*V-byte row
+// would make every warp store touch 32 sectors with 8 valid bytes each.  Every WARP owns 32 cases and
 // a private [32][W+1] tile: for a group of consecutive nodes (<= W columns of the marginal row) each
 // lane normalises its case into its tile row (conflict-free: odd row stride), then the warp streams
 // the 32 row segments to HBM, one 8*W-byte contiguous segment per store instruction.  Warps never
